@@ -3,7 +3,7 @@
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload yelp|amazon|yelp100|amazon_gcn|big]
                   [--scaling weak|strong] [--impl reference] [--check-only] [--torch-adam] [--nccl-scores]
-                  [--no-graph] [--no-cpu-baseline]
+                  [--no-graph] [--no-cpu-baseline] [--dump-outputs DIR]
 
 One "step" = one full training step of PCALayer(InterAgg3(IntraAgg x3)) on one label-balanced batch of target
 nodes: score table + pool sort (next to the choose preparation), choose, aggregate, the fused dense / loss /
@@ -594,6 +594,24 @@ def dp_self_check(model, gstep, data, params, global_batches, shards, dev, rank,
     return mean_loss, want
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, loss, model):
+    """What a caller of the timed train step ends up with after its last step: the step's loss over the global batch
+    (`loss.npy`; with several GPUs the mean of the ranks' shard losses) and every trainable parameter after the step's
+    optimizer update (`<parameter name>.npy`), float32. The inputs (graph, initial weights, batches) are seeded, so
+    two builds run with the same arguments can be compared file by file."""
+    arrays = {"loss": loss.detach().float().reshape(1)}
+    arrays.update((name, p.detach().float()) for name, p in model.named_parameters() if p.requires_grad)
+    total = sum(a.numel() * 4 for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes of outputs, more than the {DUMP_LIMIT_BYTES} allowed")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.cpu().numpy())
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -612,7 +630,14 @@ def main():
     ap.add_argument("--nccl-scores", action="store_true",
                     help="workload big: exchange the score slices with an NCCL all-gather instead of peer-memory stores")
     ap.add_argument("--nodes-per-gpu", type=int, default=1_250_000, help="workload big: rows of the CSR held per GPU")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's loss (over the global batch) and the trained "
+                         "parameters to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.check_only):
+        ap.error("--dump-outputs needs the timed steps of --impl ours")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -764,16 +789,17 @@ def main():
         return
 
     def timed(fn, first):
+        """(summed event ms of K steps, what the last step returned)"""
         evs = []
         for s in range(K):
             flush.zero_()
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
-            fn(first + s)
+            out = fn(first + s)
             e1.record()
             evs.append((e0, e1))
         torch.cuda.synchronize()
-        return sum(a.elapsed_time(b) for a, b in evs)
+        return sum(a.elapsed_time(b) for a, b in evs), out
 
     def barrier():
         torch.cuda.synchronize()
@@ -794,15 +820,25 @@ def main():
         step_device(s)
     barrier()
     sampler.start()
-    ms_dev = timed(step_device, W)
+    ms_dev, last_loss = timed(step_device, W)
     sampler.sample()
     barrier()
     ms_dev = max_over_ranks(ms_dev)
+    if args.dump_outputs:
+        # taken before the arms below train the same model further
+        if gstep is not None and gstep.overflowed():
+            raise SystemExit("--dump-outputs: a timed step overflowed its slot capacity, its outputs are incomplete")
+        loss = last_loss.detach().float().reshape(1).clone()
+        if world > 1:                  # equal shards: the mean of the ranks' losses is the loss of the global batch
+            dist.all_reduce(loss)
+            loss /= world
+        if rank == 0:
+            dump_outputs(args.dump_outputs, loss, model)
     # ---- host inputs through the step-graph API ----
     for s in range(W):
         step_host(s)
     barrier()
-    ms_graph_host = timed(step_host, W)
+    ms_graph_host, _ = timed(step_host, W)
     barrier()
     ms_graph_host = max_over_ranks(ms_graph_host)
     if gstep is not None:
@@ -831,7 +867,7 @@ def main():
             for s in range(W):
                 gstep.run_planned()
             barrier()
-            ms_plan = timed(lambda i: gstep.run_planned(), W)
+            ms_plan, _ = timed(lambda i: gstep.run_planned(), W)
             barrier()
             ms_plan = max_over_ranks(ms_plan)
             assert not gstep.overflowed()

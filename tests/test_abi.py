@@ -3,6 +3,8 @@ signature table covers exactly those symbols. No compute calls (no GPU here)."""
 import ctypes
 import os
 import re
+import subprocess
+import sys
 
 import pytest
 
@@ -55,15 +57,17 @@ def test_missing_library_fails_loudly(monkeypatch, tmp_path):
 
 
 def test_no_gpu_means_error_not_fallback():
-    import torch
-
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    from pcgnn_b200 import _lib
-    from pcgnn_b200.engine import Engine
-
-    with pytest.raises(_lib.PcgError):
-        Engine(None)
+    """Run in a child process that sees no CUDA device, so that the check also runs on a machine with a GPU."""
+    code = ("from pcgnn_b200 import _lib\n"
+            "from pcgnn_b200.engine import Engine\n"
+            "try:\n"
+            "    Engine(None)\n"
+            "except _lib.PcgError as e:\n"
+            "    print('PcgError:', e)\n")
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
+    r = subprocess.run([sys.executable, "-c", code], cwd=ROOT, env=env, capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert r.stdout.startswith("PcgError: pcgnn_b200 needs a CUDA device"), r.stdout
 
 
 def test_product_never_imports_the_oracle():
