@@ -373,6 +373,46 @@ PCG_API int pcg_score_bcast(const float* feat_rows, int64_t n_rows, int F, int64
                     int64_t row_lo, int64_t n_global, void* const* regions_host, int rank, int world,
                     uint32_t* epoch, pcg_stream_t stream);
 
+/*
+ * Evaluation pass (the batch loop of src/utils.py:298-312 and its metrics, :313-333) with every batch of the node set
+ * resident in HBM. pcg_eval_head is PCALayer's head and to_prob's sigmoid (src/model.py:38, :41-45) on one recorded
+ * batch: with entry e = *cursor % count (cursor NULL: e = 0), row i < min(B, n_total - e*B) writes
+ *   prob[c * n_total + e*B + i] = sigmoid(sum_k w_head[c,k] * emb[k,i])     emb [E,B] from pcg_tile_fwd, w_head [2,E]
+ * with k summed in order; prob is planar [2, n_total] and padding rows are not written. The cursor is not advanced
+ * (a trailing pcg_stage_indexed with bump != 0 does that).
+ *
+ * pcg_binary_metrics computes every metric of prob [2,n] (planar, as above) against int32 labels [n] (0 / 1) into
+ * out[PCG_METRICS_WORDS] doubles: prob[1] is sorted with pcg_sort_pool (labels as the pool), AUC is the Mann-Whitney
+ * statistic with average ranks for ties (NaN when one class is absent), the confusion counts take pred = 1 iff
+ * prob[1] > prob[0], F1 / recall / precision follow sklearn's zero_division=0, and the best threshold is the distinct
+ * value t of prob[1] whose cut "positive iff prob[1] >= t" has the largest macro-F1 (ties: the larger t).
+ * Deterministic (integer sums, an order-free arg-max); 0 < n < 2^31.
+ *   workspace  pcg_binary_metrics_workspace_bytes(n) bytes, 256-byte aligned
+ */
+#define PCG_METRICS_WORDS 17
+#define PCG_MT_AUC 0
+#define PCG_MT_F1 1
+#define PCG_MT_F1_MACRO 2
+#define PCG_MT_RECALL 3
+#define PCG_MT_PRECISION 4
+#define PCG_MT_RECALL_MACRO 5
+#define PCG_MT_PRECISION_MACRO 6
+#define PCG_MT_ACCURACY 7
+#define PCG_MT_GMEAN 8
+#define PCG_MT_BEST_F1_MACRO 9
+#define PCG_MT_BEST_THRESHOLD 10
+#define PCG_MT_N_POS 11
+#define PCG_MT_N_NEG 12
+#define PCG_MT_TP 13
+#define PCG_MT_FP 14
+#define PCG_MT_TN 15
+#define PCG_MT_FN 16
+PCG_API int pcg_eval_head(const float* emb, int E, int B, const float* w_head, int64_t n_total, const uint32_t* cursor,
+                  uint32_t count, float* prob, pcg_stream_t stream);
+PCG_API size_t pcg_binary_metrics_workspace_bytes(int64_t n);
+PCG_API int pcg_binary_metrics(const float* prob, const int32_t* labels, int64_t n, double* out, void* workspace,
+                       size_t workspace_bytes, pcg_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

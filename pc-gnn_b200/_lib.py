@@ -19,6 +19,10 @@ STATUS_WORDS = 12    # PCG_STATUS_WORDS
 ST_SLOTS, ST_OVERFLOW = 0, 3
 NORM_MEAN, NORM_RSQRT = 0, 1
 KB_MAX_POOL = 8192   # PCG_KB_WORDS * 32: pools up to this size use the per-item kept-pool bitmap
+# PCG_METRICS_WORDS doubles written by pcg_binary_metrics, in the order of the PCG_MT_* word indices
+METRICS_KEYS = ("auc", "f1", "f1_macro", "recall", "precision", "recall_macro", "precision_macro", "accuracy", "gmean",
+                "best_f1_macro", "best_threshold", "n_pos", "n_neg", "tp", "fp", "tn", "fn")
+METRICS_WORDS = len(METRICS_KEYS)
 
 _p = C.c_void_p
 _i = C.c_int
@@ -79,6 +83,9 @@ SIGNATURES = {
     "pcg_score_bcast": (_i, [_p, _l, _i, _l, _p, _p, _l, _l, C.POINTER(_p), _i, _i, _p, _p]),
     "pcg_pick_step": (_i, [_p, _l, _p, _l, _p, _p, _p]),
     "pcg_pick_step_philox": (_i, [_p, _l, _u64, _u64, _l, _p, _p, _p]),
+    "pcg_eval_head": (_i, [_p, _i, _i, _p, _l, _p, C.c_uint32, _p, _p]),
+    "pcg_binary_metrics_workspace_bytes": (_z, [_l]),
+    "pcg_binary_metrics": (_i, [_p, _p, _l, _p, _p, _z, _p]),
 }
 
 _lib = None

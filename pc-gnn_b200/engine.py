@@ -414,21 +414,28 @@ class Engine:
     def choose(self, targets, labels, train: bool, thresh, rho: float, cap_slots: int, *,
                entry_score=None, center_score=None, k_override=None, sorted_pool=None,
                indptr=None, indices=None, n_nodes=None, n_rel=None, max_degree=None,
-               want_dist: bool = False, phases: int = 3, sel: Selection | None = None):
+               want_dist: bool = False, phases: int = 3, sel: Selection | None = None, workspace=None):
         """Top-k filter + oversample for every (relation, target) item (``pcg_choose``).
 
         Default: the engine's resident graph, score table and pool. The keyword overrides carry the
         explicit-list calling convention of IntraAgg.forward / choose_step_* (src/layers.py:562, 633).
         Returns the Selection (and the distance buffer when want_dist).
         phases=1 runs only the score-independent preparation (callers put it on a side stream next to
-        ``score_table``), phases=2 the selection on the Selection a phases=1 call returned."""
+        ``score_table``), phases=2 the selection on the Selection a phases=1 call returned.
+        workspace: a caller-owned uint8 device buffer of at least ``pcg_choose_workspace_bytes`` bytes, initialised
+        by ``pcg_choose_workspace_init`` for this node count, used instead of the engine's shared one (which grows, and
+        so moves, with the batch size: a recorded graph that must outlive other calls brings its own)."""
         B = int(targets.shape[0])
         R = self.R if n_rel is None else n_rel
         s = sel if sel is not None else self._new_selection(B, R, cap_slots, True, False)
         maxdeg = self.max_degree if max_degree is None else max_degree
         nn_ = self.N if n_nodes is None else n_nodes
         ws_bytes = self.lib.pcg_choose_workspace_bytes(B, R, maxdeg, nn_)
-        if self._ws is None or self._ws.numel() < ws_bytes or self._ws_nodes != nn_:
+        if workspace is not None:
+            if workspace.numel() < ws_bytes:
+                raise _lib.PcgError(f"choose workspace has {workspace.numel()} bytes, this call needs {ws_bytes}")
+            ws = workspace
+        elif self._ws is None or self._ws.numel() < ws_bytes or self._ws_nodes != nn_:
             # the head of the workspace is the per-node "first occurrence" table, which the kernels expect
             # (and leave) all-0x7f: initialise it whenever the buffer or the node count behind it changes
             if self._ws is None or self._ws.numel() < ws_bytes:
@@ -436,6 +443,8 @@ class Engine:
             _lib.check(self.lib.pcg_choose_workspace_init(self._ws.data_ptr(), self._ws.numel(), nn_, _lib.stream_ptr()),
                        "pcg_choose_workspace_init")
             self._ws_nodes = nn_
+        if workspace is None:
+            ws = self._ws
         th = (C.c_double * R)(*[float(x) for x in thresh])
         use_table = entry_score is None
         if sorted_pool is None and self.sorted_pool is not None and use_table:
@@ -453,7 +462,7 @@ class Engine:
             _lib.ptr(ps), _lib.ptr(pp), _lib.ptr(pi), _lib.ptr(self.entry_pool_pos) if use_table else None, P,
             int(bool(train)), maxdeg, s.idx.data_ptr(), _lib.ptr(dist),
             cap_slots, s.slot_item.data_ptr(), s.it_slot0.data_ptr(), s.it_m.data_ptr(), s.it_base.data_ptr(),
-            s.it_done.data_ptr(), s.it_rep.data_ptr(), self._ws.data_ptr(), int(ws_bytes), s.status.data_ptr(),
+            s.it_done.data_ptr(), s.it_rep.data_ptr(), ws.data_ptr(), int(ws_bytes), s.status.data_ptr(),
             int(phases), _lib.stream_ptr())
         _lib.check(rc, "pcg_choose")
         return (s, dist) if want_dist else s

@@ -449,9 +449,10 @@ class InterAgg(nn.Module):
         return self._engine
 
     # -- forward ----------------------------------------------------------------------------
-    def _select(self, eng, targets, lab, train_flag, cap):
+    def _select(self, eng, targets, lab, train_flag, cap, *, workspace=None):
         """Score table -> pool sort -> choose (filter + oversample + union) for device-resident ids / labels and a
-        given slot capacity (layers.py:216-262, 633-738). Pure kernel launches on the current stream."""
+        given slot capacity (layers.py:216-262, 633-738). Pure kernel launches on the current stream.
+        workspace: a choose workspace of the caller's own (see ``Engine.choose``) instead of the engine's."""
         rho = self.intra_agg1.rho
         dev = eng.device
         cur = torch.cuda.current_stream(dev)
@@ -469,7 +470,7 @@ class InterAgg(nn.Module):
             side.wait_stream(cur)
             side1.wait_stream(cur)
             with torch.cuda.stream(side):
-                sel = eng.choose(targets, lab, train_flag, self.thresholds, rho, cap, phases=1)
+                sel = eng.choose(targets, lab, train_flag, self.thresholds, rho, cap, phases=1, workspace=workspace)
             with torch.cuda.stream(side1):
                 eng.sort_pool_from(pool_score)
             eng.score_table_only(self.label_clf.weight, self.label_clf.bias)
@@ -482,7 +483,7 @@ class InterAgg(nn.Module):
                 eng.fork_point()
             side.wait_stream(cur)
             with torch.cuda.stream(side):
-                sel = eng.choose(targets, lab, train_flag, self.thresholds, rho, cap, phases=1)
+                sel = eng.choose(targets, lab, train_flag, self.thresholds, rho, cap, phases=1, workspace=workspace)
             if self.score_override is not None:
                 eng.score.copy_(self.score_override)
                 eng.resort_pool()
@@ -493,7 +494,7 @@ class InterAgg(nn.Module):
             else:       # eval: no oversampling, the pool is not needed (layers.py:700-738)
                 eng.score_table_only(self.label_clf.weight, self.label_clf.bias)
             cur.wait_stream(side)
-        eng.choose(targets, lab, train_flag, self.thresholds, rho, cap, phases=2, sel=sel)
+        eng.choose(targets, lab, train_flag, self.thresholds, rho, cap, phases=2, sel=sel, workspace=workspace)
         self.last_selection = sel
         return sel
 

@@ -12,7 +12,7 @@ from __future__ import annotations
 
 import torch
 
-__all__ = ["binary_metrics"]
+__all__ = ["binary_metrics", "device_metrics"]
 
 
 def binary_metrics(prob1: torch.Tensor, pred: torch.Tensor, labels: torch.Tensor) -> dict:
@@ -50,3 +50,31 @@ def binary_metrics(prob1: torch.Tensor, pred: torch.Tensor, labels: torch.Tensor
                        (tp + tn) / float(max(n, 1)), torch.sqrt(rec1 * rec0)]).cpu().tolist()
     keys = ["auc", "f1", "f1_macro", "recall", "precision", "recall_macro", "precision_macro", "accuracy", "gmean"]
     return dict(zip(keys, out))
+
+
+def device_metrics(prob_2n: torch.Tensor, labels: torch.Tensor) -> dict:
+    """``binary_metrics`` of pred = (prob[1] > prob[0]) computed by one kernel chain (``pcg_binary_metrics``: sort,
+    counts, best threshold) plus one device->host copy. prob_2n: planar [2, n] fp32 CUDA tensor (row 1 = P(class 1));
+    labels: 0 / 1 per node. Returns python floats: the keys of ``binary_metrics`` plus best_f1_macro / best_threshold
+    (the distinct value t of prob[1] whose cut "positive iff prob[1] >= t" has the largest macro-F1, ties to the larger
+    t), n_pos, n_neg and the confusion counts tp, fp, tn, fn."""
+    from . import _lib
+
+    if prob_2n.dim() != 2 or prob_2n.shape[0] != 2 or not prob_2n.is_cuda:
+        raise ValueError(f"device_metrics: prob must be a [2, n] CUDA tensor, got {tuple(prob_2n.shape)}")
+    n = int(prob_2n.shape[1])
+    if n == 0:
+        raise ValueError("device_metrics: no nodes")
+    prob = prob_2n.to(torch.float32).contiguous()
+    y = torch.as_tensor(labels, device=prob.device).reshape(-1)
+    if y.numel() != n:
+        raise ValueError(f"device_metrics: {y.numel()} labels for {n} nodes")
+    if bool(((y != 0) & (y != 1)).any()):
+        raise ValueError("device_metrics: labels must be 0 or 1")
+    y = y.to(torch.int32).contiguous()
+    L = _lib.lib()
+    ws = torch.empty(int(L.pcg_binary_metrics_workspace_bytes(n)), dtype=torch.uint8, device=prob.device)
+    out = torch.empty(_lib.METRICS_WORDS, dtype=torch.float64, device=prob.device)
+    _lib.check(L.pcg_binary_metrics(prob.data_ptr(), y.data_ptr(), n, out.data_ptr(), ws.data_ptr(), ws.numel(),
+                                    _lib.stream_ptr()), "pcg_binary_metrics")
+    return dict(zip(_lib.METRICS_KEYS, out.cpu().tolist()))

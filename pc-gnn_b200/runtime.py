@@ -15,7 +15,7 @@ import torch
 
 from . import _lib
 
-__all__ = ["GraphedTrainStep"]
+__all__ = ["GraphedTrainStep", "GraphedEvalPass", "pack_eval_plan"]
 
 
 class GraphedTrainStep:
@@ -380,3 +380,181 @@ class GraphedTrainStep:
     def plan(engine, batches, thresholds, rho) -> int:
         """Slot capacity covering every batch of an epoch plan (host arithmetic on CSR offsets)."""
         return max(engine.slots_bound(np.asarray(n, dtype=np.int32), thresholds, rho, True) for n in batches)
+
+
+# -- evaluation: the test loop of utils.py:298-333 over a whole node set, recorded ------------------------------------
+def pack_eval_plan(nodes, batch_size: int) -> np.ndarray:
+    """A node set as an int32 [n_entries, batch_size] plan in the given order. The last entry is padded with copies of
+    its own first id: pcg_choose folds repeated targets onto their first occurrence (``it_rep``), so the padding adds
+    no choose or aggregate work, and the rows it produces are never written out."""
+    B = int(batch_size)
+    if B <= 0:
+        raise ValueError(f"batch_size must be positive, got {batch_size}")
+    ids = np.asarray(nodes, dtype=np.int64).reshape(-1)
+    n = ids.shape[0]
+    if n == 0:
+        raise ValueError("an evaluation pass needs at least one node")
+    if ids.min() < 0 or ids.max() > np.iinfo(np.int32).max:
+        raise ValueError("node ids must lie in [0, 2^31)")
+    n_entries = -(-n // B)
+    plan = np.empty((n_entries, B), dtype=np.int32)
+    flat = plan.reshape(-1)
+    flat[:n] = ids
+    flat[n:] = ids[(n_entries - 1) * B]
+    return plan
+
+
+class GraphedEvalPass:
+    """Scores a whole node set (validation, test, all nodes) with PCALayer and computes its metrics on the device:
+    ``run()`` is n_entries replays of one recorded batch graph, one replay of a metrics graph and one host wait.
+
+    The ids are uploaded once as a plan of ``batch_size``-wide entries; the batch graph fetches entry ``cursor``
+    (``InterAgg.stage_in``), runs the eval-mode selection (score table, choose) with a choose workspace of its own,
+    the aggregation, the fused dense kernel and the head + sigmoid (``pcg_eval_head``) into a planar [2, n]
+    probability buffer, then advances the cursor with a copy of the batch's overflow word into a per-entry array.
+    The metrics graph runs ``pcg_binary_metrics`` and copies the result block and the overflow words to pinned memory.
+
+    Replays read the current parameter values, so in-place updates (optimizer steps) need nothing; a parameter or the
+    feature table moving to new storage, or new thresholds, re-record on the next ``run()``. There is no torch
+    fallback: models, tables, graphs and shapes the recorded path does not cover raise ``PcgError``."""
+
+    def __init__(self, model, nodes, labels, batch_size: int, cap_slots: int | None = None):
+        from .layers import InterAgg
+        from .model import PCALayer
+
+        if not isinstance(model, PCALayer) or not isinstance(getattr(model, "inter1", None), InterAgg):
+            raise _lib.PcgError(f"GraphedEvalPass runs PCALayer over an InterAgg, not {type(model).__name__}")
+        plan = pack_eval_plan(nodes, batch_size)
+        y = np.asarray(labels).reshape(-1)
+        n = int(np.asarray(nodes).reshape(-1).shape[0])
+        if y.shape[0] != n:
+            raise ValueError(f"{y.shape[0]} labels for {n} nodes")
+        if not np.isin(y, (0, 1)).all():
+            raise ValueError("labels must be 0 or 1")
+        self.model, self.B, self.n = model, int(batch_size), n
+        self.n_entries = int(plan.shape[0])
+        inter = model.inter1
+        eng = inter.engine()
+        self._state()                                  # refusals before any allocation
+        dev = eng.device
+        L = _lib.lib()
+        self._plan = torch.from_numpy(plan).to(dev)
+        self._labels = torch.from_numpy(y.astype(np.int32)).to(dev)
+        self._nodes = torch.empty(self.B, dtype=torch.int32, device=dev)
+        self._cursor = torch.zeros(1, dtype=torch.int32, device=dev)
+        self._prob = torch.empty((2, n), dtype=torch.float32, device=dev)
+        # [metrics (doubles) | overflow word of every entry]: one block, one copy to the host
+        W = _lib.METRICS_WORDS
+        self._res = torch.zeros(2 * W + self.n_entries, dtype=torch.int32, device=dev)
+        self._out = self._res[:2 * W].view(torch.float64)
+        self._ovf = self._res[2 * W:]
+        self._pin = torch.zeros(self._res.numel(), dtype=torch.int32, pin_memory=True)
+        self._pin_np = self._pin.numpy()
+        self._mws = torch.empty(int(L.pcg_binary_metrics_workspace_bytes(n)), dtype=torch.uint8, device=dev)
+        # the pass's own choose workspace, sized for its batch and initialised once: the engine's shared one is
+        # reallocated when a larger batch comes along, which recorded graphs must never see
+        ws_bytes = int(L.pcg_choose_workspace_bytes(self.B, eng.R, eng.max_degree, eng.N))
+        self._ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+        _lib.check(L.pcg_choose_workspace_init(self._ws.data_ptr(), ws_bytes, eng.N, _lib.stream_ptr()),
+                   "pcg_choose_workspace_init")
+        if cap_slots is None:
+            rho = float(inter.intra_agg1.rho)
+            cap_slots = max(eng.slots_bound(e, inter.thresholds, rho, False) for e in plan)
+        self.cap_slots = int(cap_slots)
+        self._done = torch.cuda.Event()
+        self._key = None
+        self.g_batch = self.g_metrics = None
+        self.captures = 0
+
+    def _params(self):
+        inter = self.model.inter1
+        return [self.model.weight, inter.label_clf.weight, inter.label_clf.bias, inter.weight] + \
+            [ia.weight for ia in inter.intra_aggs()]
+
+    def _state(self):
+        """What the recording bakes in (parameter and feature-table addresses, thresholds), after the refusals."""
+        import torch.nn as nn
+
+        from .layers import _feature_table
+
+        inter = self.model.inter1
+        eng = inter.engine()
+        table = _feature_table(inter.features, eng.N_global, eng.device)
+        if table.requires_grad:
+            raise _lib.PcgError("GraphedEvalPass: the feature table is trainable (the recorded path has no gradient to it)")
+        if eng.graph.partitioned or eng.score_group is not None or eng._bcast is not None or inter.scores_external:
+            raise _lib.PcgError("GraphedEvalPass: row-partitioned graphs and exchanged score tables are not supported")
+        if self.model.weight.shape[0] != 2 or not isinstance(inter.label_clf, nn.Linear) or inter.label_clf.bias is None:
+            raise _lib.PcgError("GraphedEvalPass: needs a two-class head and label_clf = nn.Linear with a bias")
+        params = self._params()
+        if any(not p.is_contiguous() or p.dtype != torch.float32 or p.device != eng.device for p in params):
+            raise _lib.PcgError("GraphedEvalPass: parameters must be contiguous fp32 tensors on the engine's device")
+        eng.set_features(table)
+        E = int(inter.weight.shape[1])
+        if not eng.tile_supported(self.B, eng.R, E):
+            raise _lib.PcgError(f"GraphedEvalPass: pcg_tile_supported rejects B={self.B} R={eng.R} F={eng.F} E={E}")
+        return tuple(p.data_ptr() for p in params) + (eng.feat.data_ptr(),), tuple(float(t) for t in inter.thresholds)
+
+    def _record(self):
+        from .stepgraph import StepGraphCache
+
+        L = _lib.lib()
+        inter = self.model.inter1
+        eng = inter.engine()
+        p = [q.detach() for q in self._params()]
+        head, w_inter, w_intra = p[0], p[3], p[4:]
+        E, B, nb = int(w_inter.shape[1]), self.B, self.n_entries
+        cur = self._cursor.data_ptr()
+
+        def batch():
+            inter.stage_in = (self._plan.data_ptr(), self._nodes.data_ptr(), B * 4, cur, nb, B * 4)
+            sel = inter._select(eng, self._nodes, None, False, self.cap_slots, workspace=self._ws)
+            agg = eng.aggregate(sel, copy_dups=False)
+            out, _, _ = eng.tile_fwd(self._nodes, agg, sel.it_rep, w_intra, w_inter, None, None, False)
+            _lib.check(L.pcg_eval_head(out.data_ptr(), E, B, head.data_ptr(), self.n, cur, nb, self._prob.data_ptr(),
+                                       _lib.stream_ptr()), "pcg_eval_head")
+            _lib.check(L.pcg_stage_indexed(sel.status[_lib.ST_OVERFLOW:].data_ptr(), self._ovf.data_ptr(), 4, cur, nb, 0, 4,
+                                           1, _lib.stream_ptr()), "pcg_stage_indexed")
+            return sel
+
+        def metrics():
+            _lib.check(L.pcg_binary_metrics(self._prob.data_ptr(), self._labels.data_ptr(), self.n, self._out.data_ptr(),
+                                            self._mws.data_ptr(), self._mws.numel(), _lib.stream_ptr()),
+                       "pcg_binary_metrics")
+            _lib.check(L.pcg_stage(self._res.data_ptr(), _lib.host_device_ptr(self._pin), self._res.numel() * 4,
+                                   _lib.stream_ptr()), "pcg_stage")
+
+        last = inter.last_selection
+        try:
+            self.g_batch, _ = StepGraphCache._capture(batch, eng.device)
+            self.g_metrics, _ = StepGraphCache._capture(metrics, eng.device)
+        finally:
+            inter.stage_in = None
+            inter.last_selection = last
+        self.captures += 1
+
+    def run(self) -> dict:
+        """Scores every node and returns the metrics as python floats: the keys of ``metrics.binary_metrics`` (pred =
+        prob[1] > prob[0], as utils.test) plus best_f1_macro, best_threshold, n_pos, n_neg and tp / fp / tn / fn.
+        Raises PcgError when a batch needed more slots than ``cap_slots`` (its scores would be incomplete)."""
+        key = self._state()
+        if key != self._key:
+            self.g_batch = self.g_metrics = None
+            self._record()
+            self._key = key
+        self._cursor.zero_()
+        for _ in range(self.n_entries):
+            self.g_batch.replay()
+        self.g_metrics.replay()
+        self._done.record(torch.cuda.current_stream(self._prob.device))
+        self._done.synchronize()
+        W = _lib.METRICS_WORDS
+        bad = np.flatnonzero(self._pin_np[2 * W:])
+        if bad.size:
+            raise _lib.PcgError(f"GraphedEvalPass: {bad.size} of {self.n_entries} batches needed more than cap_slots="
+                                f"{self.cap_slots} slots (first: entry {int(bad[0])}); build the pass with a larger capacity")
+        return dict(zip(_lib.METRICS_KEYS, self._pin_np[:2 * W].view(np.float64).tolist()))
+
+    def probs(self) -> torch.Tensor:
+        """[n, 2] view of the last run's probabilities (to_prob's first output), in the caller's node order."""
+        return self._prob.t()
