@@ -375,11 +375,14 @@ PCG_API int pcg_score_bcast(const float* feat_rows, int64_t n_rows, int F, int64
 
 /*
  * Evaluation pass (the batch loop of src/utils.py:298-312 and its metrics, :313-333) with every batch of the node set
- * resident in HBM. pcg_eval_head is PCALayer's head and to_prob's sigmoid (src/model.py:38, :41-45) on one recorded
- * batch: with entry e = *cursor % count (cursor NULL: e = 0), row i < min(B, n_total - e*B) writes
- *   prob[c * n_total + e*B + i] = sigmoid(sum_k w_head[c,k] * emb[k,i])     emb [E,B] from pcg_tile_fwd, w_head [2,E]
- * with k summed in order; prob is planar [2, n_total] and padding rows are not written. The cursor is not advanced
- * (a trailing pcg_stage_indexed with bump != 0 does that).
+ * resident in HBM. pcg_eval_head is the two-class head and to_prob's output on one recorded batch: with entry
+ * e = *cursor % count (cursor NULL: e = 0) and l_c = sum_k w_head[c,k] * emb[k,i] (k summed in order 0..E-1), row
+ * i < min(B, n_total - e*B) writes
+ *   mode 0: prob[c * n_total + e*B + i] = sigmoid(l_c)     PCALayer (src/model.py:38, :41-45), GCN (src/graphsage.py:154-178)
+ *   mode 1: prob[c * n_total + e*B + i] = (l_c - m) - log(exp(l_0 - m) + exp(l_1 - m)),  m = max(l_0, l_1)
+ *           the log_softmax of GraphSage.to_prob (src/graphsage.py:16-39, over dim 1)
+ * emb [E,B] from pcg_tile_fwd or pcg_encoder_fwd, w_head [2,E]; prob is planar [2, n_total] and padding rows are not
+ * written. The cursor is not advanced (a trailing pcg_stage_indexed with bump != 0 does that).
  *
  * pcg_binary_metrics computes every metric of prob [2,n] (planar, as above) against int32 labels [n] (0 / 1) into
  * out[PCG_METRICS_WORDS] doubles: prob[1] is sorted with pcg_sort_pool (labels as the pool), AUC is the Mann-Whitney
@@ -407,8 +410,8 @@ PCG_API int pcg_score_bcast(const float* feat_rows, int64_t n_rows, int F, int64
 #define PCG_MT_FP 14
 #define PCG_MT_TN 15
 #define PCG_MT_FN 16
-PCG_API int pcg_eval_head(const float* emb, int E, int B, const float* w_head, int64_t n_total, const uint32_t* cursor,
-                  uint32_t count, float* prob, pcg_stream_t stream);
+PCG_API int pcg_eval_head(const float* emb, int E, int B, const float* w_head, int mode, int64_t n_total,
+                  const uint32_t* cursor, uint32_t count, float* prob, pcg_stream_t stream);
 PCG_API size_t pcg_binary_metrics_workspace_bytes(int64_t n);
 PCG_API int pcg_binary_metrics(const float* prob, const int32_t* labels, int64_t n, double* out, void* workspace,
                        size_t workspace_bytes, pcg_stream_t stream);

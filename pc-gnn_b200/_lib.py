@@ -83,7 +83,7 @@ SIGNATURES = {
     "pcg_score_bcast": (_i, [_p, _l, _i, _l, _p, _p, _l, _l, C.POINTER(_p), _i, _i, _p, _p]),
     "pcg_pick_step": (_i, [_p, _l, _p, _l, _p, _p, _p]),
     "pcg_pick_step_philox": (_i, [_p, _l, _u64, _u64, _l, _p, _p, _p]),
-    "pcg_eval_head": (_i, [_p, _i, _i, _p, _l, _p, C.c_uint32, _p, _p]),
+    "pcg_eval_head": (_i, [_p, _i, _i, _p, _i, _l, _p, C.c_uint32, _p, _p]),
     "pcg_binary_metrics_workspace_bytes": (_z, [_l]),
     "pcg_binary_metrics": (_i, [_p, _p, _l, _p, _p, _z, _p]),
 }

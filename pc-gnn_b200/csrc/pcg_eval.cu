@@ -1,15 +1,17 @@
-// Evaluation pass on the device: PCALayer's head + sigmoid into a whole-set probability buffer, and the binary
-// metrics of src/utils.py:298-333 (AUC, F1, recall, precision, ...) plus a best-threshold macro-F1, computed where
-// the probabilities live. Deterministic: integer sums and an order-free arg-max only (no floating-point atomics).
+// Evaluation pass on the device: the two-class head + sigmoid (PCALayer, GCN) or log-softmax (GraphSage) into a
+// whole-set probability buffer, and the binary metrics of src/utils.py:298-333 (AUC, F1, recall, precision, ...) plus
+// a best-threshold macro-F1, computed where the probabilities live. Deterministic: integer sums and an order-free
+// arg-max only (no floating-point atomics).
 #include <math.h>
 
 #include "pcg_common.cuh"
 
 // ------------------------------------------------------------------------------- head
-// prob[c * n_total + e*B + i] = sigmoid(sum_k w[c,k] * emb[k,i]) for the rows of plan entry e = *cursor % count that
-// exist (padding rows of the last entry are not written). One thread per row, k summed in order 0..E-1.
+// l_c = sum_k w[c,k] * emb[k,i] for the rows of plan entry e = *cursor % count that exist (padding rows of the last
+// entry are not written), k summed in order 0..E-1, one thread per row. mode 0: prob[c * n_total + e*B + i] =
+// sigmoid(l_c); mode 1: log_softmax(l)_c = (l_c - m) - log(exp(l_0 - m) + exp(l_1 - m)) with m = max(l_0, l_1).
 __global__ void __launch_bounds__(256) k_eval_head(const float* __restrict__ emb, int E, int B, const float* __restrict__ w,
-                                                   int64_t n_total, const uint32_t* cursor, uint32_t count,
+                                                   int mode, int64_t n_total, const uint32_t* cursor, uint32_t count,
                                                    float* __restrict__ prob) {
     extern __shared__ float sw[];
     for (int k = threadIdx.x; k < 2 * E; k += blockDim.x) sw[k] = w[k];
@@ -24,18 +26,26 @@ __global__ void __launch_bounds__(256) k_eval_head(const float* __restrict__ emb
         a0 = fmaf(sw[k], x, a0);
         a1 = fmaf(sw[E + k], x, a1);
     }
-    prob[base + i] = 1.f / (1.f + expf(-a0));
-    prob[n_total + base + i] = 1.f / (1.f + expf(-a1));
+    if (mode == 0) {
+        prob[base + i] = 1.f / (1.f + expf(-a0));
+        prob[n_total + base + i] = 1.f / (1.f + expf(-a1));
+    } else {
+        const float m = fmaxf(a0, a1);
+        const float lse = logf(expf(a0 - m) + expf(a1 - m));
+        prob[base + i] = (a0 - m) - lse;
+        prob[n_total + base + i] = (a1 - m) - lse;
+    }
 }
 
-extern "C" int pcg_eval_head(const float* emb, int E, int B, const float* w_head, int64_t n_total, const uint32_t* cursor,
-                             uint32_t count, float* prob, pcg_stream_t stream_) {
+extern "C" int pcg_eval_head(const float* emb, int E, int B, const float* w_head, int mode, int64_t n_total,
+                             const uint32_t* cursor, uint32_t count, float* prob, pcg_stream_t stream_) {
     cudaStream_t stream = (cudaStream_t)stream_;
     PCG_REQUIRE(emb && w_head && prob, "pcg_eval_head: null pointer");
     PCG_REQUIRE(E > 0 && E <= 4096 && B > 0 && n_total > 0, "pcg_eval_head: need 0 < E <= 4096, B > 0, n_total > 0");
+    PCG_REQUIRE(mode == 0 || mode == 1, "pcg_eval_head: mode must be 0 (sigmoid) or 1 (log-softmax), got %d", mode);
     PCG_REQUIRE(!cursor || count > 0, "pcg_eval_head: a plan cursor needs count > 0");
-    k_eval_head<<<(B + 255) / 256, 256, (size_t)E * 2 * sizeof(float), stream>>>(emb, E, B, w_head, n_total, cursor, count,
-                                                                                  prob);
+    k_eval_head<<<(B + 255) / 256, 256, (size_t)E * 2 * sizeof(float), stream>>>(emb, E, B, w_head, mode, n_total, cursor,
+                                                                                  count, prob);
     return pcg_check_launch("pcg_eval_head");
 }
 

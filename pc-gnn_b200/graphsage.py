@@ -47,6 +47,11 @@ class _EncoderFn(torch.autograd.Function):
         return None, None, None, (None if sink is not None else d_w)
 
 
+def _encoder_fits(enc, eng) -> bool:
+    """Whether pcg_encoder_fwd / _bwd take this encoder: the weight and a tile of targets fit in shared memory."""
+    return (enc.weight.shape[1] * (eng.ldf + 33) + enc.weight.numel()) * 4 <= 190 * 1024
+
+
 def _encode(enc, nodes, with_self):
     """Shared forward of Encoder / GCNEncoder: aggregate, then the encoder kernel when the feature table is frozen
     (the reference's setup) or the torch ops when it trains."""
@@ -56,7 +61,7 @@ def _encode(enc, nodes, with_self):
     table = getattr(enc.features, "weight", None)
     native = (eng is not None and isinstance(table, torch.Tensor) and not table.requires_grad and neigh_feats.is_cuda
               and agg_mod.last_targets is not None and neigh_feats.shape[0] > 0 and neigh_feats.shape[1] == eng.F
-              and (enc.weight.shape[1] * (eng.ldf + 33) + enc.weight.numel()) * 4 <= 190 * 1024)
+              and _encoder_fits(enc, eng))
     if native:
         full = agg_mod.last_agg          # [B, ldf] as the kernel wrote it (row stride ldf)
         return _EncoderFn.apply(eng, full, agg_mod.last_targets if with_self else None, enc.weight)

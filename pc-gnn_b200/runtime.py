@@ -383,10 +383,14 @@ class GraphedTrainStep:
 
 
 # -- evaluation: the test loop of utils.py:298-333 over a whole node set, recorded ------------------------------------
-def pack_eval_plan(nodes, batch_size: int) -> np.ndarray:
+def pack_eval_plan(nodes, batch_size: int, indptr=None) -> np.ndarray:
     """A node set as an int32 [n_entries, batch_size] plan in the given order. The last entry is padded with copies of
     its own first id: pcg_choose folds repeated targets onto their first occurrence (``it_rep``), so the padding adds
-    no choose or aggregate work, and the rows it produces are never written out."""
+    no choose or aggregate work, and the rows it produces are never written out.
+
+    indptr: CSR row offsets of a one-relation graph (the GCN / GraphSAGE baselines). pcg_select_all does not fold
+    repeated targets, so every padding row aggregates its node's whole row; with indptr the padding repeats the set's
+    node with the shortest row (the first such node in the given order) instead."""
     B = int(batch_size)
     if B <= 0:
         raise ValueError(f"batch_size must be positive, got {batch_size}")
@@ -400,31 +404,60 @@ def pack_eval_plan(nodes, batch_size: int) -> np.ndarray:
     plan = np.empty((n_entries, B), dtype=np.int32)
     flat = plan.reshape(-1)
     flat[:n] = ids
-    flat[n:] = ids[(n_entries - 1) * B]
+    if indptr is None:
+        flat[n:] = ids[(n_entries - 1) * B]
+    else:
+        ip = np.asarray(indptr, dtype=np.int64)
+        if ids.max() >= ip.shape[0] - 1:
+            raise ValueError(f"node id {int(ids.max())} is not a row of the graph ({ip.shape[0] - 1} rows)")
+        flat[n:] = ids[np.argmin(ip[ids + 1] - ip[ids])]
     return plan
 
 
-class GraphedEvalPass:
-    """Scores a whole node set (validation, test, all nodes) with PCALayer and computes its metrics on the device:
-    ``run()`` is n_entries replays of one recorded batch graph, one replay of a metrics graph and one host wait.
+def _baseline_parts(model):
+    """(aggregator, add_self, with_self, head mode) of graphsage.GCN over GCNEncoder(GCNAggregator) or GraphSage over
+    Encoder(MeanAggregator); None for PCALayer over an InterAgg; PcgError for anything else."""
+    from .graphsage import GCN, Encoder, GCNAggregator, GCNEncoder, GraphSage, MeanAggregator
+    from .layers import InterAgg
+    from .model import PCALayer
 
-    The ids are uploaded once as a plan of ``batch_size``-wide entries; the batch graph fetches entry ``cursor``
+    if isinstance(model, PCALayer) and isinstance(getattr(model, "inter1", None), InterAgg):
+        return None
+    enc = getattr(model, "enc", None)
+    agg = getattr(enc, "aggregator", None)
+    if isinstance(model, GCN) and isinstance(enc, GCNEncoder) and isinstance(agg, GCNAggregator):
+        return agg, True, False, 0
+    if isinstance(model, GraphSage) and isinstance(enc, Encoder) and isinstance(agg, MeanAggregator):
+        return agg, bool(agg.gcn), not enc.gcn, 1
+    raise _lib.PcgError("GraphedEvalPass runs PCALayer over an InterAgg, GCN over GCNEncoder(GCNAggregator) or "
+                        f"GraphSage over Encoder(MeanAggregator), not {type(model).__name__}")
+
+
+class GraphedEvalPass:
+    """Scores a whole node set (validation, test, all nodes) with PCALayer, graphsage.GCN or graphsage.GraphSage and
+    computes its metrics on the device: ``run()`` is n_entries replays of one recorded batch graph, one replay of a
+    metrics graph and one host wait.
+
+    The ids are uploaded once as a plan of ``batch_size``-wide entries. PCALayer's batch graph fetches entry ``cursor``
     (``InterAgg.stage_in``), runs the eval-mode selection (score table, choose) with a choose workspace of its own,
-    the aggregation, the fused dense kernel and the head + sigmoid (``pcg_eval_head``) into a planar [2, n]
-    probability buffer, then advances the cursor with a copy of the batch's overflow word into a per-entry array.
-    The metrics graph runs ``pcg_binary_metrics`` and copies the result block and the overflow words to pinned memory.
+    the aggregation, the fused dense kernel and the head + sigmoid (``pcg_eval_head``). The baselines' batch graph
+    fetches the entry (``pcg_stage_indexed``), selects the targets' whole rows (``pcg_select_all``, with the target
+    itself where the aggregator adds it), aggregates them with the aggregator's norm, runs ``pcg_encoder_fwd`` (with
+    the self rows for ``Encoder(gcn=False)``) and the head + to_prob's sigmoid (GCN) or log-softmax (GraphSage); their
+    plans are padded with the set's lowest-degree node (``pack_eval_plan``'s indptr). Either writes a planar [2, n]
+    buffer, then advances the cursor with a copy of the batch's overflow word into a per-entry array. The metrics graph
+    runs ``pcg_binary_metrics`` and copies the result block and the overflow words to pinned memory.
 
     Replays read the current parameter values, so in-place updates (optimizer steps) need nothing; a parameter or the
-    feature table moving to new storage, or new thresholds, re-record on the next ``run()``. There is no torch
-    fallback: models, tables, graphs and shapes the recorded path does not cover raise ``PcgError``."""
+    feature table moving to new storage, new thresholds (PCALayer) or another engine (an aggregator bound to another
+    graph) re-record on the next ``run()``. The modules' own state (``last_selection``, ``cap_slots_hint``, ...) is
+    left alone. There is no torch fallback: models, tables, graphs and shapes the recorded path does not cover raise
+    ``PcgError``."""
 
     def __init__(self, model, nodes, labels, batch_size: int, cap_slots: int | None = None):
-        from .layers import InterAgg
-        from .model import PCALayer
-
-        if not isinstance(model, PCALayer) or not isinstance(getattr(model, "inter1", None), InterAgg):
-            raise _lib.PcgError(f"GraphedEvalPass runs PCALayer over an InterAgg, not {type(model).__name__}")
-        plan = pack_eval_plan(nodes, batch_size)
+        self._homo = _baseline_parts(model)
+        eng = model.inter1.engine() if self._homo is None else self._homo[0]._get_engine()
+        plan = pack_eval_plan(nodes, batch_size, None if self._homo is None else eng.graph.indptr[:eng.N + 1])
         y = np.asarray(labels).reshape(-1)
         n = int(np.asarray(nodes).reshape(-1).shape[0])
         if y.shape[0] != n:
@@ -433,11 +466,10 @@ class GraphedEvalPass:
             raise ValueError("labels must be 0 or 1")
         self.model, self.B, self.n = model, int(batch_size), n
         self.n_entries = int(plan.shape[0])
-        inter = model.inter1
-        eng = inter.engine()
         self._state()                                  # refusals before any allocation
         dev = eng.device
         L = _lib.lib()
+        self._plan_host = plan
         self._plan = torch.from_numpy(plan).to(dev)
         self._labels = torch.from_numpy(y.astype(np.int32)).to(dev)
         self._nodes = torch.empty(self.B, dtype=torch.int32, device=dev)
@@ -451,32 +483,53 @@ class GraphedEvalPass:
         self._pin = torch.zeros(self._res.numel(), dtype=torch.int32, pin_memory=True)
         self._pin_np = self._pin.numpy()
         self._mws = torch.empty(int(L.pcg_binary_metrics_workspace_bytes(n)), dtype=torch.uint8, device=dev)
-        # the pass's own choose workspace, sized for its batch and initialised once: the engine's shared one is
-        # reallocated when a larger batch comes along, which recorded graphs must never see
-        ws_bytes = int(L.pcg_choose_workspace_bytes(self.B, eng.R, eng.max_degree, eng.N))
-        self._ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
-        _lib.check(L.pcg_choose_workspace_init(self._ws.data_ptr(), ws_bytes, eng.N, _lib.stream_ptr()),
-                   "pcg_choose_workspace_init")
-        if cap_slots is None:
-            rho = float(inter.intra_agg1.rho)
-            cap_slots = max(eng.slots_bound(e, inter.thresholds, rho, False) for e in plan)
-        self.cap_slots = int(cap_slots)
+        self._cap_arg = cap_slots
+        if self._homo is None:
+            inter = model.inter1
+            # the pass's own choose workspace, sized for its batch and initialised once: the engine's shared one is
+            # reallocated when a larger batch comes along, which recorded graphs must never see
+            ws_bytes = int(L.pcg_choose_workspace_bytes(self.B, eng.R, eng.max_degree, eng.N))
+            self._ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+            _lib.check(L.pcg_choose_workspace_init(self._ws.data_ptr(), ws_bytes, eng.N, _lib.stream_ptr()),
+                       "pcg_choose_workspace_init")
+            if cap_slots is None:
+                rho = float(inter.intra_agg1.rho)
+                cap_slots = max(eng.slots_bound(e, inter.thresholds, rho, False) for e in plan)
+            self.cap_slots = int(cap_slots)
+        else:
+            self.cap_slots = self._baseline_capacity()
         self._done = torch.cuda.Event()
         self._key = None
         self.g_batch = self.g_metrics = None
         self.captures = 0
 
+    def _baseline_capacity(self) -> int:
+        """The caller's capacity, else exactly the largest per-entry slot demand on the aggregator's current graph."""
+        if self._cap_arg is not None:
+            return int(self._cap_arg)
+        return max(self._homo[0].slots_bound(e) for e in self._plan_host)
+
     def _params(self):
+        if self._homo is not None:
+            return [self.model.weight, self.model.enc.weight]
         inter = self.model.inter1
         return [self.model.weight, inter.label_clf.weight, inter.label_clf.bias, inter.weight] + \
             [ia.weight for ia in inter.intra_aggs()]
 
+    @staticmethod
+    def _check_params(params, eng):
+        if any(not p.is_contiguous() or p.dtype != torch.float32 or p.device != eng.device for p in params):
+            raise _lib.PcgError("GraphedEvalPass: parameters must be contiguous fp32 tensors on the engine's device")
+
     def _state(self):
-        """What the recording bakes in (parameter and feature-table addresses, thresholds), after the refusals."""
+        """What the recording bakes in (parameter and feature-table addresses, thresholds / engine), after the
+        refusals."""
         import torch.nn as nn
 
         from .layers import _feature_table
 
+        if self._homo is not None:
+            return self._state_baseline()
         inter = self.model.inter1
         eng = inter.engine()
         table = _feature_table(inter.features, eng.N_global, eng.device)
@@ -487,23 +540,47 @@ class GraphedEvalPass:
         if self.model.weight.shape[0] != 2 or not isinstance(inter.label_clf, nn.Linear) or inter.label_clf.bias is None:
             raise _lib.PcgError("GraphedEvalPass: needs a two-class head and label_clf = nn.Linear with a bias")
         params = self._params()
-        if any(not p.is_contiguous() or p.dtype != torch.float32 or p.device != eng.device for p in params):
-            raise _lib.PcgError("GraphedEvalPass: parameters must be contiguous fp32 tensors on the engine's device")
+        self._check_params(params, eng)
         eng.set_features(table)
         E = int(inter.weight.shape[1])
         if not eng.tile_supported(self.B, eng.R, E):
             raise _lib.PcgError(f"GraphedEvalPass: pcg_tile_supported rejects B={self.B} R={eng.R} F={eng.F} E={E}")
         return tuple(p.data_ptr() for p in params) + (eng.feat.data_ptr(),), tuple(float(t) for t in inter.thresholds)
 
+    def _state_baseline(self):
+        from .graphsage import _encoder_fits
+        from .layers import _feature_table
+
+        agg, _, with_self, _ = self._homo
+        enc = self.model.enc
+        eng = agg._get_engine()
+        table = _feature_table(agg.features, eng.N, eng.device)
+        if table.requires_grad:
+            raise _lib.PcgError("GraphedEvalPass: the feature table is trainable (the recorded path has no gradient to it)")
+        if eng.graph.partitioned or eng.R != 1:
+            raise _lib.PcgError("GraphedEvalPass: the baselines need an unpartitioned one-relation graph (row-partitioned "
+                                f"or multi-relation graphs are not supported; this one has {eng.R} relations)")
+        if self.model.weight.shape[0] != 2:
+            raise _lib.PcgError("GraphedEvalPass: needs a two-class head")
+        params = self._params()
+        self._check_params(params, eng)
+        eng.set_features(table)
+        E, f_in = int(enc.weight.shape[0]), eng.F * (2 if with_self else 1)
+        if enc.weight.shape[1] != f_in or self.model.weight.shape[1] != E or not _encoder_fits(enc, eng):
+            raise _lib.PcgError(f"GraphedEvalPass: pcg_encoder_fwd does not take an encoder weight of shape "
+                                f"{tuple(enc.weight.shape)} (F={eng.F}, head {tuple(self.model.weight.shape)})")
+        return tuple(p.data_ptr() for p in params) + (eng.feat.data_ptr(),), eng
+
     def _record(self):
         from .stepgraph import StepGraphCache
 
-        L = _lib.lib()
+        if self._homo is not None:
+            return self._record_baseline()
         inter = self.model.inter1
         eng = inter.engine()
         p = [q.detach() for q in self._params()]
         head, w_inter, w_intra = p[0], p[3], p[4:]
-        E, B, nb = int(w_inter.shape[1]), self.B, self.n_entries
+        B, nb = self.B, self.n_entries
         cur = self._cursor.data_ptr()
 
         def batch():
@@ -511,31 +588,60 @@ class GraphedEvalPass:
             sel = inter._select(eng, self._nodes, None, False, self.cap_slots, workspace=self._ws)
             agg = eng.aggregate(sel, copy_dups=False)
             out, _, _ = eng.tile_fwd(self._nodes, agg, sel.it_rep, w_intra, w_inter, None, None, False)
-            _lib.check(L.pcg_eval_head(out.data_ptr(), E, B, head.data_ptr(), self.n, cur, nb, self._prob.data_ptr(),
-                                       _lib.stream_ptr()), "pcg_eval_head")
-            _lib.check(L.pcg_stage_indexed(sel.status[_lib.ST_OVERFLOW:].data_ptr(), self._ovf.data_ptr(), 4, cur, nb, 0, 4,
-                                           1, _lib.stream_ptr()), "pcg_stage_indexed")
+            self._head_and_overflow(out, head, 0, sel)
             return sel
-
-        def metrics():
-            _lib.check(L.pcg_binary_metrics(self._prob.data_ptr(), self._labels.data_ptr(), self.n, self._out.data_ptr(),
-                                            self._mws.data_ptr(), self._mws.numel(), _lib.stream_ptr()),
-                       "pcg_binary_metrics")
-            _lib.check(L.pcg_stage(self._res.data_ptr(), _lib.host_device_ptr(self._pin), self._res.numel() * 4,
-                                   _lib.stream_ptr()), "pcg_stage")
 
         last = inter.last_selection
         try:
             self.g_batch, _ = StepGraphCache._capture(batch, eng.device)
-            self.g_metrics, _ = StepGraphCache._capture(metrics, eng.device)
+            self.g_metrics, _ = StepGraphCache._capture(self._metrics, eng.device)
         finally:
             inter.stage_in = None
             inter.last_selection = last
         self.captures += 1
 
+    def _record_baseline(self):
+        from .stepgraph import StepGraphCache
+
+        agg, add_self, with_self, mode = self._homo
+        eng = agg._get_engine()
+        head, w_enc = [q.detach() for q in self._params()]
+        B, nb = self.B, self.n_entries
+        self.cap_slots = self._baseline_capacity()
+
+        def batch():
+            eng.stage(self._plan.data_ptr(), self._nodes.data_ptr(), B * 4, self._cursor.data_ptr(), nb, B * 4)
+            sel = eng.select_all(self._nodes, add_self, self.cap_slots, agg._norm)
+            emb = eng.encoder_fwd(eng.aggregate(sel), w_enc, self._nodes if with_self else None)
+            self._head_and_overflow(emb, head, mode, sel)
+            return sel
+
+        self.g_batch, _ = StepGraphCache._capture(batch, eng.device)
+        self.g_metrics, _ = StepGraphCache._capture(self._metrics, eng.device)
+        self.captures += 1
+
+    def _head_and_overflow(self, emb, head, mode, sel):
+        """(recorded) pcg_eval_head into the entry's rows of the probability buffer, then the batch's overflow word into
+        the entry's slot of the overflow array, advancing the cursor."""
+        L = _lib.lib()
+        cur, nb = self._cursor.data_ptr(), self.n_entries
+        _lib.check(L.pcg_eval_head(emb.data_ptr(), int(emb.shape[0]), self.B, head.data_ptr(), mode, self.n, cur, nb,
+                                   self._prob.data_ptr(), _lib.stream_ptr()), "pcg_eval_head")
+        _lib.check(L.pcg_stage_indexed(sel.status[_lib.ST_OVERFLOW:].data_ptr(), self._ovf.data_ptr(), 4, cur, nb, 0, 4, 1,
+                                       _lib.stream_ptr()), "pcg_stage_indexed")
+
+    def _metrics(self):
+        L = _lib.lib()
+        _lib.check(L.pcg_binary_metrics(self._prob.data_ptr(), self._labels.data_ptr(), self.n, self._out.data_ptr(),
+                                        self._mws.data_ptr(), self._mws.numel(), _lib.stream_ptr()), "pcg_binary_metrics")
+        _lib.check(L.pcg_stage(self._res.data_ptr(), _lib.host_device_ptr(self._pin), self._res.numel() * 4,
+                               _lib.stream_ptr()), "pcg_stage")
+
     def run(self) -> dict:
         """Scores every node and returns the metrics as python floats: the keys of ``metrics.binary_metrics`` (pred =
         prob[1] > prob[0], as utils.test) plus best_f1_macro, best_threshold, n_pos, n_neg and tp / fp / tn / fn.
+        The metrics are computed on ``probs()`` as they are: for GraphSage, log-probabilities, so ``best_threshold``
+        is a log-probability there (pred and AUC are unchanged by the log).
         Raises PcgError when a batch needed more slots than ``cap_slots`` (its scores would be incomplete)."""
         key = self._state()
         if key != self._key:
@@ -556,5 +662,6 @@ class GraphedEvalPass:
         return dict(zip(_lib.METRICS_KEYS, self._pin_np[:2 * W].view(np.float64).tolist()))
 
     def probs(self) -> torch.Tensor:
-        """[n, 2] view of the last run's probabilities (to_prob's first output), in the caller's node order."""
+        """[n, 2] view of the last run's to_prob output (PCALayer: its first output), in the caller's node order:
+        probabilities for PCALayer and GCN, log-probabilities for GraphSage."""
         return self._prob.t()
