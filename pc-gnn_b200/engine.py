@@ -358,26 +358,11 @@ class Engine:
         dst = torch.empty(B, dtype=torch.int32, device=self.device)
         return self._pin.upload(host, dst), host
 
-    def slots_bound(self, host_targets, thresh, rho, train, *, k_override=None) -> int:
-        """Upper bound of the slots a batch needs, from the host copy of the CSR offsets (every
+    def slots_bound(self, host_targets, thresh, rho, train) -> int:
+        """Upper bound of the slots a batch needs: the graph's per-node choose demand summed over the host ids (every
         target counted as positive when training, since labels may live on the device)."""
-        t = host_targets.astype(np.int64) - self.row_lo
-        total = 0
-        for r in range(self.R):
-            rows = r * self.N + t
-            d = self.graph.indptr[rows + 1] - self.graph.indptr[rows]
-            if k_override is not None:
-                c = np.asarray(k_override[r * len(t):(r + 1) * len(t)], dtype=np.int64)
-            else:
-                c = np.ceil(d * float(thresh[r])).astype(np.int64)
-            k = np.where(d > c + 1, c, d)
-            o = np.minimum((c * float(rho)).astype(np.int64), self.P) if train else 0
-            total += int(((k + o + _lib.SLOT - 1) // _lib.SLOT).sum())
-        return max(total, 1)
-
-    def slots_bound_all(self, B: int) -> int:
-        """Select-all bound without host ids: every item as long as the longest row."""
-        return B * self.R * max(1, (self.max_degree + _lib.SLOT - 1) // _lib.SLOT)
+        demand = self.graph.choose_slot_demand(thresh, rho, self.P, train)
+        return max(int(demand[np.asarray(host_targets, dtype=np.int64) - self.row_lo].sum()), 1)
 
     # ------------------------------------------------------------------ kernels
     def _new_selection(self, B, R, cap_slots, with_sel_idx, with_extra):

@@ -16,7 +16,18 @@ from __future__ import annotations
 
 import numpy as np
 
-__all__ = ["RelGraph", "csr_from_edges", "adj_lists_from_csr"]
+from ._lib import SLOT
+
+__all__ = ["RelGraph", "csr_from_edges", "adj_lists_from_csr", "item_slots"]
+
+
+def item_slots(d, c, rho, P, train):
+    """Slots the choose kernel gives items with row lengths ``d`` and kept counts ``c`` (int64 arrays): k kept ids, plus
+    the oversampled pool members when training, in whole slots. Mirrors ``item_counts()`` in csrc/pcg_common.cuh, with
+    every target counted as positive."""
+    k = np.where(d > c + 1, c, d)
+    o = np.minimum((c * float(rho)).astype(np.int64), P) if train else 0
+    return (k + o + SLOT - 1) // SLOT
 
 
 def csr_from_edges(n_nodes: int, src, dst, *, symmetric: bool = True, self_loops: bool = True):
@@ -192,6 +203,26 @@ class RelGraph:
     def degrees(self, r: int):
         n = self.n_nodes
         return np.diff(self.indptr[r * n:(r + 1) * n + 1])
+
+    # ---- slot demand: per-node tables behind the host's slot capacities ----
+    def choose_slot_demand(self, thresholds, rho, P, train):
+        """Read-only int64 [n_nodes]: the slots the choose kernel can give a target, summed over relations, with
+        ``c = ceil(d * thresholds[r])`` (``item_slots``). A batch's capacity is the sum over its targets."""
+        thr = tuple(float(t) for t in thresholds)
+        return self._slot_demand((thr, float(rho), int(P), bool(train)),
+                                 lambda r, d: item_slots(d, np.ceil(d * thr[r]).astype(np.int64), rho, P, train))
+
+    def select_all_slot_demand(self):
+        """Read-only int64 [n_nodes]: the slots the select-all kernel can give a target, summed over relations: each row
+        in whole slots, and one slot for an empty row (it may still take the target itself)."""
+        return self._slot_demand(None, lambda r, d: np.maximum((d + SLOT - 1) // SLOT, 1))
+
+    def _slot_demand(self, key, per_relation):
+        memo = self.__dict__.setdefault("_slot_demand_memo", {})     # lazily: from_device_csr skips __init__
+        if key not in memo:
+            memo[key] = sum(per_relation(r, self.degrees(r)) for r in range(self.n_rel))
+            memo[key].flags.writeable = False
+        return memo[key]
 
     def union(self):
         """Single-relation graph whose rows are the union over relations — the

@@ -121,11 +121,9 @@ class _RowAggregator(nn.Module):
             self._engine = Engine(self._graph, dev)
         return self._engine
 
-    def _run(self, eng, targets, degrees, add_self, n_table=None):
+    def _run(self, eng, targets, cap, add_self, n_table=None):
         table = _feature_table(self.features, eng.N if n_table is None else n_table, eng.device)
         eng.set_features(table)
-        cap = int(np.maximum((degrees + _lib.SLOT - 1) // _lib.SLOT, 1).sum()) if degrees is not None \
-            else int(self.cap_slots_hint)
         sel = eng.select_all(targets, add_self, cap, self._norm)
         self.last_selection = sel
         agg = _AggregateFn.apply(table, eng, sel, table.shape[1]) if table.requires_grad else eng.aggregate(sel)
@@ -138,18 +136,14 @@ class _RowAggregator(nn.Module):
         eng = self._get_engine()
         targets, host = eng.upload_targets(nodes)
         if self.cap_slots_hint is not None:
-            return self._run(eng, targets, None, add_self)
-        if host is None:
-            host = targets.cpu().numpy()
-        t = host.astype(np.int64)
-        return self._run(eng, targets, eng.graph.indptr[t + 1] - eng.graph.indptr[t], add_self)
+            cap = int(self.cap_slots_hint)
+        else:
+            cap = self.slots_bound(targets.cpu().numpy() if host is None else host)
+        return self._run(eng, targets, cap, add_self)
 
     def slots_bound(self, nodes) -> int:
-        """Slot capacity that covers a batch of node ids (host arithmetic on the CSR offsets)."""
-        g = self._get_engine().graph
-        t = np.asarray(nodes, dtype=np.int64)
-        d = g.indptr[t + 1] - g.indptr[t]
-        return int(np.maximum((d + _lib.SLOT - 1) // _lib.SLOT, 1).sum())
+        """Slot capacity that covers a batch of node ids (the graph's per-node select-all demand, summed)."""
+        return int(self._get_engine().graph.select_all_slot_demand()[np.asarray(nodes, dtype=np.int64)].sum())
 
     def _aggregate_lists(self, nodes, to_neighs, add_self):
         """Explicit neighbour sets (stand-alone aggregator use, or sub-sampled rows): a one-off graph
@@ -164,8 +158,8 @@ class _RowAggregator(nn.Module):
         eng = Engine(RelGraph.from_adj_lists([rows], max(n_ids, len(rows))), self._device())
         eng.strict_rows = False            # graph rows are batch positions, not node ids
         targets = torch.arange(len(rows), dtype=torch.int32, device=eng.device)
-        d = np.fromiter((len(rows[i]) for i in range(len(rows))), dtype=np.int64, count=len(rows))
-        return self._run(eng, targets, d, False, n_table=n_ids)
+        cap = int(eng.graph.select_all_slot_demand()[:len(rows)].sum())
+        return self._run(eng, targets, cap, False, n_table=n_ids)
 
 
 class MeanAggregator(_RowAggregator):

@@ -29,7 +29,7 @@ from torch.nn import init
 
 from . import _lib
 from .engine import Engine
-from .graph import RelGraph
+from .graph import RelGraph, item_slots
 
 __all__ = ["InterAgg1", "InterAgg3", "InterAgg5", "InterAgg", "IntraAgg", "choose_step_neighs",
            "choose_step_test", "HeadLossFn", "TrainStepFn"]
@@ -331,9 +331,8 @@ def _choose_explicit(eng, center_scores, center_labels, neigh_scores, neighs_lis
         pool_score = torch.as_tensor(minor_scores).detach().to(dev, torch.float32).reshape(-1, 2)[:, 0].contiguous()
         P = int(pool.shape[0])
         sorted_pool = eng.sort_pool(pool, pool_score)
-    kk = np.where(lens > k_list + 1, k_list, lens)
-    oo = np.minimum((k_list * float(sample_rate)).astype(np.int64), P) if train else np.zeros_like(kk)
-    cap = int(((kk + oo + _lib.SLOT - 1) // _lib.SLOT).sum()) + 1
+    oo = np.minimum((k_list * float(sample_rate)).astype(np.int64), P) if train else np.zeros_like(k_list)
+    cap = int(item_slots(lens, k_list, sample_rate, P, train).sum()) + 1
     targets = torch.arange(B, dtype=torch.int32, device=dev)
     labels = _as_device_labels(center_labels, dev) if train else None
     sel, dist = eng.choose(targets, labels, train, [0.5], float(sample_rate), cap, entry_score=entry_score,
@@ -510,10 +509,8 @@ class InterAgg(nn.Module):
         lab = _as_device_labels(labels, dev) if train_flag else None
         if self.cap_slots_hint is not None:
             cap = int(self.cap_slots_hint)
-        elif host is not None:
-            cap = eng.slots_bound(host, self.thresholds, rho, train_flag)
         else:
-            cap = eng.slots_bound(targets.cpu().numpy(), self.thresholds, rho, train_flag)
+            cap = eng.slots_bound(targets.cpu().numpy() if host is None else host, self.thresholds, rho, train_flag)
         return eng, table, targets, lab, self._select(eng, targets, lab, train_flag, cap)
 
     def graphs(self):

@@ -378,8 +378,8 @@ class GraphedTrainStep:
 
     @staticmethod
     def plan(engine, batches, thresholds, rho) -> int:
-        """Slot capacity covering every batch of an epoch plan (host arithmetic on CSR offsets)."""
-        return max(engine.slots_bound(np.asarray(n, dtype=np.int32), thresholds, rho, True) for n in batches)
+        """Slot capacity covering every batch of an epoch plan (the largest ``Engine.slots_bound`` of a batch)."""
+        return max(engine.slots_bound(n, thresholds, rho, True) for n in batches)
 
 
 # -- evaluation: the test loop of utils.py:298-333 over a whole node set, recorded ------------------------------------
@@ -493,8 +493,7 @@ class GraphedEvalPass:
             _lib.check(L.pcg_choose_workspace_init(self._ws.data_ptr(), ws_bytes, eng.N, _lib.stream_ptr()),
                        "pcg_choose_workspace_init")
             if cap_slots is None:
-                rho = float(inter.intra_agg1.rho)
-                cap_slots = max(eng.slots_bound(e, inter.thresholds, rho, False) for e in plan)
+                cap_slots = max(eng.slots_bound(e, inter.thresholds, inter.intra_agg1.rho, False) for e in plan)
             self.cap_slots = int(cap_slots)
         else:
             self.cap_slots = self._baseline_capacity()

@@ -8,8 +8,8 @@ into static buffers and replays: the caller's loop stays exactly the reference's
 
 What a cached graph bakes in, and how each is kept honest:
   * parameter / feature-table addresses  -> compared on every call, a change re-records the graph
-  * the slot capacity of the selection    -> a per-node bound table (host) is summed over the batch's ids on every
-                                             call; a batch that needs more re-records with a larger capacity
+  * the slot capacity of the selection    -> the batch's training-mode ``Engine.slots_bound`` (it covers eval mode too)
+                                             on every call; a batch that needs more re-records with a larger capacity
   * lambda, rho, thresholds               -> part of the cache key
 Training graphs hold the whole step behind the upload (score table, pool sort, choose, aggregate, the fused dense
 / loss / gradient kernels); the returned loss carries an autograd node whose backward hands out the gradients the
@@ -54,30 +54,10 @@ class StepGraphCache:
     def __init__(self, inter):
         self.inter = inter
         self.slots = {}
-        self.node_cap = None          # int32 [N]: slots a node's items can need (all relations, positive, train)
-        self._node_cap_key = None
         self.stage_nodes = None
         self.stage_labels = None
         self.replays = 0
         self.captures = 0
-
-    # ------------------------------------------------------------------ capacity
-    def _bound_table(self, eng):
-        inter = self.inter
-        rho = float(inter.intra_agg1.rho)
-        key = (tuple(float(t) for t in inter.thresholds), rho, eng.P)
-        if self.node_cap is None or self._node_cap_key != key:
-            g = eng.graph
-            tot = np.zeros(g.n_nodes, dtype=np.int64)
-            for r in range(g.n_rel):
-                d = g.degrees(r).astype(np.int64)
-                c = np.ceil(d * float(inter.thresholds[r])).astype(np.int64)
-                k = np.where(d > c + 1, c, d)
-                o = np.minimum((c * rho).astype(np.int64), eng.P)
-                tot += (k + o + _lib.SLOT - 1) // _lib.SLOT
-            self.node_cap = tot
-            self._node_cap_key = key
-        return self.node_cap
 
     def _ids(self, nodes):
         if isinstance(nodes, torch.Tensor):
@@ -92,7 +72,8 @@ class StepGraphCache:
                 and eng.score_group is None and eng._bcast is None and not eng.graph.partitioned
                 and eng.grad_sink is None and not table.requires_grad)
 
-    def _slot(self, key, ptrs, need, build):
+    def _slot(self, eng, key, ptrs, host, build):
+        need = eng.slots_bound(host, self.inter.thresholds, self.inter.intra_agg1.rho, True)
         slot = self.slots.get(key)
         if slot is not None and (slot.ptrs != ptrs or slot.cap < need):
             del self.slots[key]
@@ -153,7 +134,6 @@ class StepGraphCache:
                  [ia.weight for ia in inter.intra_aggs()]
         ptrs = tuple(p.data_ptr() for p in params) + (eng.feat.data_ptr(),)
         key = ("train", B, float(lam), float(inter.intra_agg1.rho), tuple(float(t) for t in inter.thresholds))
-        need = int(self._bound_table(eng)[host].sum())
         dev = eng.device
 
         def build(slot):
@@ -180,7 +160,7 @@ class StepGraphCache:
 
             slot.graph, (slot.out, slot.sel) = self._capture(fn, dev)
 
-        slot = self._slot(key, ptrs, need, build)
+        slot = self._slot(eng, key, ptrs, host, build)
         self._upload(slot, host, nodes, labels, dev)
         slot.graph.replay()
         self.replays += 1
@@ -201,7 +181,6 @@ class StepGraphCache:
         params = [inter.label_clf.weight, inter.label_clf.bias, inter.weight] + [ia.weight for ia in inter.intra_aggs()]
         ptrs = tuple(p.data_ptr() for p in params) + (eng.feat.data_ptr(),)
         key = ("infer", B, bool(train_flag), float(inter.intra_agg1.rho), tuple(float(t) for t in inter.thresholds))
-        need = int(self._bound_table(eng)[host].sum())
         dev = eng.device
 
         def build(slot):
@@ -218,7 +197,7 @@ class StepGraphCache:
 
             slot.graph, (slot.out, slot.sel) = self._capture(fn, dev)
 
-        slot = self._slot(key, ptrs, need, build)
+        slot = self._slot(eng, key, ptrs, host, build)
         self._upload(slot, host, nodes, labels if train_flag else None, dev)
         slot.graph.replay()
         self.replays += 1

@@ -46,17 +46,13 @@ def test_c4_last_entry_slot_demand():
     """C4 (amazon union graph, idx_rest, B = 1024): the last entry holds 64 nodes and 960 padding rows. Every padding
     row costs the slots of its node's whole row, so the set's shortest row (306 entries) keeps that entry at about half
     the slots of a full one; the entry's first id as the padding made it cost as much as a full entry."""
-    from pcgnn_b200 import _lib
     from pcgnn_b200.synth import make_graph
 
     d = make_graph("amazon", seed=72)
     ip = d.homo.indptr
     nodes = np.asarray(d.idx_rest)
     B = 1024
-
-    def slots(ids):
-        deg = ip[ids.astype(np.int64) + 1] - ip[ids.astype(np.int64)]
-        return int(np.maximum((deg + _lib.SLOT - 1) // _lib.SLOT, 1).sum())
+    slots = lambda ids: int(d.homo.select_all_slot_demand()[ids].sum())
 
     plan = pack_eval_plan(nodes, B, ip)
     assert plan.shape == (6, B) and len(nodes) == 5184

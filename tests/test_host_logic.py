@@ -7,7 +7,8 @@ import sys
 import numpy as np
 import pytest
 
-from oracle import ref_harness as H
+from oracle import c_oracle, ref_harness as H
+from pcgnn_b200 import _lib
 from pcgnn_b200.graph import RelGraph, adj_lists_from_csr, csr_from_edges
 from pcgnn_b200.synth import make_graph
 
@@ -63,26 +64,43 @@ def test_pick_weights_and_replay_equal_random_choices():
     assert port.pick_step_replay(d.idx_train, w, u) == want
 
 
-def test_slots_bound_is_an_upper_bound_of_the_oracle_sizes():
-    from oracle import c_oracle
-    from pcgnn_b200 import _lib
+def _oracle_slots(graph, score, nodes, pool, train):
+    sp, _ = c_oracle.choose(graph, score, nodes, np.ones(len(nodes), bool), pool=pool, train=train)
+    return int(((np.diff(sp) + _lib.SLOT - 1) // _lib.SLOT).sum())
 
+
+def test_slots_bound_is_an_upper_bound_of_the_oracle_sizes():
     d = make_graph("tiny", seed=5, dup_feature_frac=0.2)
     rng = np.random.default_rng(0)
     nodes = rng.choice(d.idx_train, 100)
     score = rng.normal(size=d.feat.shape[0]).astype(np.float32)
     pool = sorted(d.train_pos)
-    sp, _ = c_oracle.choose(d.graph, score, nodes, np.ones(100, bool), pool=pool, train=True)
-    need = int(((np.diff(sp) + _lib.SLOT - 1) // _lib.SLOT).sum())
-    # same arithmetic as Engine.slots_bound, without constructing an Engine (no GPU here)
-    total = 0
-    for r in range(3):
-        deg = d.graph.degrees(r)[nodes]
-        c = np.ceil(deg * 0.5).astype(np.int64)
-        k = np.where(deg > c + 1, c, deg)
-        o = np.minimum((c * 0.5).astype(np.int64), len(pool))
-        total += int(((k + o + _lib.SLOT - 1) // _lib.SLOT).sum())
+    need = _oracle_slots(d.graph, score, nodes, pool, True)
+    total = int(d.graph.choose_slot_demand([0.5] * 3, 0.5, len(pool), True)[nodes].sum())
     assert total >= need
+
+
+def test_choose_slot_demand_is_the_oracle_demand_in_eval_mode():
+    """Unique targets, rows of several slots: in eval mode an item fills exactly the slots of its k kept ids. Train mode
+    reserves k + o slots per item before the union with the pool, so there the demand is only a bound."""
+    d = make_graph("amazon", seed=72)
+    rng = np.random.default_rng(0)
+    nodes = rng.choice(np.unique(d.idx_train), 256, replace=False)
+    score = rng.normal(size=d.feat.shape[0]).astype(np.float32)
+    pool = sorted(d.train_pos)
+    for train in (False, True):
+        demand = d.graph.choose_slot_demand([0.5] * 3, 0.5, len(pool), train)
+        got, need = int(demand[nodes].sum()), _oracle_slots(d.graph, score, nodes, pool, train)
+        assert (got >= need) if train else (got == need), (train, got, need)
+        assert d.graph.choose_slot_demand([0.5] * 3, 0.5, len(pool), train) is demand        # memoised
+
+
+def test_select_all_slot_demand_is_whole_rows_in_slots():
+    """Per node, each relation's row in 64-id slots, and one slot for an empty row (it may take the target itself)."""
+    deg = ([0, 1, 63, 64, 65, 128, 129, 0], [0, 0, 1, 64, 0, 200, 1, 65])
+    ips = [np.concatenate([[0], np.cumsum(dr)]) for dr in deg]
+    g = RelGraph(8, ips, [np.zeros(ip[-1], dtype=np.int32) for ip in ips])
+    assert g.select_all_slot_demand().tolist() == [1 + 1, 1 + 1, 1 + 1, 1 + 1, 2 + 1, 2 + 4, 3 + 1, 1 + 2]
 
 
 def test_shim_routes_reference_imports_to_this_package():
