@@ -608,10 +608,14 @@ __global__ void __launch_bounds__(TILE_NT, 1) k_tile(TileP p) {
 //   job 0      dW'  [K2p, E] = cat^T  @ dZ          (cat padded: [B, K2p])
 //   job 1 + r  dW_r'[2Fp, E] = [self | agg_r]^T @ dH_r
 //   job R + 1  the tiles' small partial sums (d W_head, d W_clf, d b_clf, losses) added in tile order
-// One cluster of S CTAs per 64 x 64 output tile; CTA `rank` of the cluster multiplies batch slice `rank` (16-byte
-// cp.async operand tiles, two stages), leaves its partial tile in its own shared memory, and after one cluster
-// barrier every CTA adds 64/S rows of the tile over the S CTAs through distributed shared memory in rank order
-// (deterministic) and stores the rows of the unpadded gradient. No global partials, no atomics, no tickets.
+// The grid is a flat list of clusters of S CTAs: first one cluster for job R + 1, then one per W x W output block of
+// jobs 0..R (built from each job's real row count, so no CTA is launched only to return). CTA `rank` of a cluster
+// multiplies batch slice `rank` (one fmaf chain per output element over the slice's rows in ascending order, from 0),
+// leaves its partial block in its own shared memory, and after one cluster barrier every CTA adds W/S rows of the
+// block over the S CTAs through distributed shared memory in rank order (deterministic) and stores the rows of the
+// unpadded gradient. No global partials, no atomics, no tickets. The block width W only decides which CTA computes an
+// element, never how: every W gives the same bits. The operand slice comes in 16-byte cp.async chunks of WG_KC rows:
+// all at once behind one wait when the slice fits the CTA's buffers, else through a two-stage ring.
 // (Round 1: k_gemm_v to global split partials + a separate k_dense_reduce launch.)
 struct WgP {
     const float* cat; int64_t ldcat;        // [B, K2p]
@@ -629,22 +633,36 @@ __device__ __forceinline__ void cp_async16_(float* smem_dst, const float* gsrc, 
     asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(d), "l"(gsrc), "r"(bytes) : "memory");
 }
 
-#define WG_KC 32
-#define WG_LD 68
-__global__ void __launch_bounds__(256) k_wgrad(WgP p) {
-    __shared__ __align__(16) float smw[2 * 2 * WG_KC * WG_LD];   // As[2][KC][LD] | Bs[2][KC][LD]; later the C tile [64][LD]
-    float (*As)[WG_KC][WG_LD] = reinterpret_cast<float (*)[WG_KC][WG_LD]>(smw);
-    float (*Bs)[WG_KC][WG_LD] = reinterpret_cast<float (*)[WG_KC][WG_LD]>(smw + 2 * WG_KC * WG_LD);
+#define WG_KC 32                            // batch rows per operand chunk
+#define WG_BUF_BYTES (48 * 1024)            // operand buffers of one CTA
+
+template <int W> struct WgShape {
+    static constexpr int T = W / 16;                          // a thread's T x T accumulators (16 x 16 threads)
+    static constexpr int LD = W + 4;
+    static constexpr int CHUNK = 2 * WG_KC * LD;              // floats: A rows | B rows
+    static constexpr int NBUF = WG_BUF_BYTES / (CHUNK * 4);   // chunks held at once
+    static_assert(NBUF >= 2 && W * LD <= NBUF * CHUNK, "wgrad buffers");
+};
+
+template <int T> __device__ __forceinline__ void ld_vec(float (&v)[T], const float* s) {
+    if constexpr (T == 4) { const float4 x = *reinterpret_cast<const float4*>(s); v[0] = x.x; v[1] = x.y; v[2] = x.z; v[3] = x.w; }
+    else { static_assert(T == 2, "T"); const float2 x = *reinterpret_cast<const float2*>(s); v[0] = x.x; v[1] = x.y; }
+}
+
+template <int W>   // 3 CTAs per SM: room for 80 registers, which k_wgrad<64> needs to run without spills
+__global__ void __launch_bounds__(256, 3) k_wgrad(WgP p) {
+    using SH = WgShape<W>;
+    constexpr int T = SH::T, LD = SH::LD, NBUF = SH::NBUF;
+    __shared__ __align__(16) float smw[NBUF * SH::CHUNK];   // chunk c: A [KC][LD] | B [KC][LD]; later the C block [W][LD]
     float* Cs = smw;
     cg::cluster_group cl = cg::this_cluster();
     const int tid = threadIdx.x, ty = tid >> 4, tx = tid & 15;
     const int S = p.S;
-    const int job = blockIdx.z / S, split = blockIdx.z - job * S;       // split == rank in the cluster (cluster dims 1,1,S)
+    const int cluster = blockIdx.x / S, split = blockIdx.x - cluster * S;   // split == rank in the cluster (dims S,1,1)
     const int E = p.E, RE = p.R * p.E;
-    if (job == p.R + 1) {
-        // ---- small gradients: sum over the tiles in tile order. CTA `split` owns a slice of the record's columns;
-        // thread (g, c): column c, tiles [g*T/8, (g+1)*T/8) in order; the 8 group sums are added in group order.
-        if (blockIdx.x != 0 || blockIdx.y != 0) return;
+    if (cluster == 0) {
+        // ---- job R + 1, small gradients: sum over the tiles in tile order. CTA `split` owns a slice of the record's
+        // columns; thread (g, c): column c, tiles [g*n/8, (g+1)*n/8) of n in order; the 8 group sums are added in group order.
         grid_dependency_wait();
         float* red = smw;                                              // [8][32] group sums, then the column totals
         const int n_real = 4 + 2 * E + 2 * p.F;
@@ -679,21 +697,27 @@ __global__ void __launch_bounds__(256) k_wgrad(WgP p) {
         }
         return;
     }
+    // ---- which output block: job 0 has ceil(K2p / W) row blocks, jobs 1..R ceil(2Fp / W) each, all ceil(E / W) columns
     const int K2p = p.Fp + p.R * p.E;
+    const int ncb = (E + W - 1) / W, nb0 = (K2p + W - 1) / W * ncb, nb1 = (2 * p.Fp + W - 1) / W * ncb;
+    int blk = cluster - 1, job = 0;
+    if (blk >= nb0) { blk -= nb0; job = 1 + blk / nb1; blk -= (job - 1) * nb1; }
     const int rows = job == 0 ? K2p : 2 * p.Fp;
-    const int m0 = blockIdx.x * 64, n0 = blockIdx.y * 64;
-    if (m0 >= rows) return;                 // the whole cluster leaves (same tile for all its CTAs)
+    const int m0 = blk / ncb * W, n0 = (blk % ncb) * W;
     pcg_launch_dependents();                // the exchange + Adam kernel may queue up
     grid_dependency_wait();
     const int per = (p.B + S - 1) / S;
     const int kb = min(p.B, split * per), ke = min(p.B, kb + per);
     const int nt = (ke - kb + WG_KC - 1) / WG_KC;
-    auto issue = [&](int t) {
-        const int buf = t & 1, k0 = kb + t * WG_KC;
+    // chunk t (rows kb + t*KC ..) -> buffer `buf`; rows past the slice are zero-filled (they add fmaf(0, 0, acc) == acc)
+    auto issue = [&](int t, int buf) {
+        float* As = smw + buf * SH::CHUNK;
+        float* Bs = As + WG_KC * LD;
+        const int k0 = kb + t * WG_KC;
 #pragma unroll
-        for (int j = 0; j < 2; ++j) {
+        for (int j = 0; j < WG_KC * W / 4 / 256; ++j) {
             const int c = tid + 256 * j;
-            const int kk = c >> 4, q4 = (c & 15) * 4;
+            const int kk = c / (W / 4), q4 = (c % (W / 4)) * 4;
             const int i = k0 + kk;
             const bool krow = i < ke;
             const int m = m0 + q4, n = n0 + q4;
@@ -709,43 +733,57 @@ __global__ void __launch_bounds__(256) k_wgrad(WgP p) {
             }
             const float* b = p.dz;
             if (bb > 0) b = job == 0 ? p.dz + (int64_t)i * E + n : p.dh + (int64_t)i * RE + (job - 1) * E + n;
-            cp_async16_(&As[buf][kk][q4], a, ba);
-            cp_async16_(&Bs[buf][kk][q4], b, bb);
+            cp_async16_(As + kk * LD + q4, a, ba);
+            cp_async16_(Bs + kk * LD + q4, b, bb);
         }
     };
-    float acc[4][4];
+    float acc[T][T];
 #pragma unroll
-    for (int a = 0; a < 4; ++a)
+    for (int a = 0; a < T; ++a)
 #pragma unroll
-        for (int b = 0; b < 4; ++b) acc[a][b] = 0.f;
-    if (nt > 0) issue(0);
-    asm volatile("cp.async.commit_group;" ::: "memory");
-    for (int t = 0; t < nt; ++t) {
-        if (t + 1 < nt) issue(t + 1);
-        asm volatile("cp.async.commit_group;" ::: "memory");
-        asm volatile("cp.async.wait_group 1;" ::: "memory");
-        __syncthreads();
-        const int cur = t & 1;
+        for (int b = 0; b < T; ++b) acc[a][b] = 0.f;
+    auto chunk_fma = [&](int buf) {
+        const float* As = smw + buf * SH::CHUNK;
+        const float* Bs = As + WG_KC * LD;
 #pragma unroll
         for (int kk = 0; kk < WG_KC; ++kk) {
-            const float4 a4 = *reinterpret_cast<const float4*>(&As[cur][kk][ty * 4]);
-            const float4 b4 = *reinterpret_cast<const float4*>(&Bs[cur][kk][tx * 4]);
-            acc[0][0] = fmaf(a4.x, b4.x, acc[0][0]); acc[0][1] = fmaf(a4.x, b4.y, acc[0][1]);
-            acc[0][2] = fmaf(a4.x, b4.z, acc[0][2]); acc[0][3] = fmaf(a4.x, b4.w, acc[0][3]);
-            acc[1][0] = fmaf(a4.y, b4.x, acc[1][0]); acc[1][1] = fmaf(a4.y, b4.y, acc[1][1]);
-            acc[1][2] = fmaf(a4.y, b4.z, acc[1][2]); acc[1][3] = fmaf(a4.y, b4.w, acc[1][3]);
-            acc[2][0] = fmaf(a4.z, b4.x, acc[2][0]); acc[2][1] = fmaf(a4.z, b4.y, acc[2][1]);
-            acc[2][2] = fmaf(a4.z, b4.z, acc[2][2]); acc[2][3] = fmaf(a4.z, b4.w, acc[2][3]);
-            acc[3][0] = fmaf(a4.w, b4.x, acc[3][0]); acc[3][1] = fmaf(a4.w, b4.y, acc[3][1]);
-            acc[3][2] = fmaf(a4.w, b4.z, acc[3][2]); acc[3][3] = fmaf(a4.w, b4.w, acc[3][3]);
-        }
-        __syncthreads();
-    }
-    asm volatile("cp.async.wait_group 0;" ::: "memory");
-    // this CTA's partial tile -> its shared memory (the operand buffers are free behind the loop's last barrier)
+            float av[T], bv[T];
+            ld_vec<T>(av, As + kk * LD + ty * T);
+            ld_vec<T>(bv, Bs + kk * LD + tx * T);
 #pragma unroll
-    for (int a = 0; a < 4; ++a)
-        *reinterpret_cast<float4*>(Cs + (ty * 4 + a) * WG_LD + tx * 4) = make_float4(acc[a][0], acc[a][1], acc[a][2], acc[a][3]);
+            for (int a = 0; a < T; ++a)
+#pragma unroll
+                for (int b = 0; b < T; ++b) acc[a][b] = fmaf(av[a], bv[b], acc[a][b]);
+        }
+    };
+    if (NBUF > 2 && nt <= NBUF) {
+        // the whole slice fits: every copy in flight at once, one wait (with two buffers the ring below does the same)
+        for (int t = 0; t < nt; ++t) issue(t, t);
+        asm volatile("cp.async.commit_group;" ::: "memory");
+        asm volatile("cp.async.wait_group 0;" ::: "memory");
+        __syncthreads();
+        for (int t = 0; t < nt; ++t) chunk_fma(t);
+        __syncthreads();
+    } else {
+        issue(0, 0);
+        asm volatile("cp.async.commit_group;" ::: "memory");
+        for (int t = 0; t < nt; ++t) {
+            if (t + 1 < nt) issue(t + 1, (t + 1) & 1);
+            asm volatile("cp.async.commit_group;" ::: "memory");
+            asm volatile("cp.async.wait_group 1;" ::: "memory");
+            __syncthreads();
+            chunk_fma(t & 1);
+            __syncthreads();
+        }
+        asm volatile("cp.async.wait_group 0;" ::: "memory");
+    }
+    // this CTA's partial block -> its shared memory (the operand buffers are free behind the last barrier)
+#pragma unroll
+    for (int a = 0; a < T; ++a) {
+        float* c = Cs + (ty * T + a) * LD + tx * T;
+        if constexpr (T == 4) *reinterpret_cast<float4*>(c) = make_float4(acc[a][0], acc[a][1], acc[a][2], acc[a][3]);
+        else *reinterpret_cast<float2*>(c) = make_float2(acc[a][0], acc[a][1]);
+    }
     cl.sync();
     // map a padded row to the row of the real gradient (or -1 for a pad row)
     auto real_row = [&](int m) -> int {
@@ -755,16 +793,16 @@ __global__ void __launch_bounds__(256) k_wgrad(WgP p) {
         return q < p.F ? p.F + q : -1;
     };
     float* grad = p.grad[job];
-    const int rpc = 64 / S;                  // rows of the tile this CTA adds up (S in {1, 2, 4, 8})
-    for (int idx = tid; idx < rpc * 16; idx += 256) {
-        const int lr = idx >> 4, q4 = (idx & 15) * 4;
+    const int rpc = W / S;                   // rows of the block this CTA adds up (S in {1, 2, 4, 8})
+    for (int idx = tid; idx < rpc * (W / 4); idx += 256) {
+        const int lr = idx / (W / 4), q4 = (idx % (W / 4)) * 4;
         const int ml = split * rpc + lr, m = m0 + ml, n = n0 + q4;
         const int rr = m < rows ? real_row(m) : -1;
         if (rr < 0 || n >= E) continue;
         float4 v[8];
 #pragma unroll
         for (int q = 0; q < 8; ++q)
-            v[q] = q < S ? *reinterpret_cast<const float4*>(cl.map_shared_rank(Cs, q) + ml * WG_LD + q4) : make_float4(0.f, 0.f, 0.f, 0.f);
+            v[q] = q < S ? *reinterpret_cast<const float4*>(cl.map_shared_rank(Cs, q) + ml * LD + q4) : make_float4(0.f, 0.f, 0.f, 0.f);
         float4 sacc = v[0];
 #pragma unroll
         for (int q = 1; q < 8; ++q) if (q < S) f4_add(sacc, v[q]);
@@ -772,7 +810,7 @@ __global__ void __launch_bounds__(256) k_wgrad(WgP p) {
         if (((uintptr_t)g & 15) == 0) *reinterpret_cast<float4*>(g) = sacc;
         else { g[0] = sacc.x; g[1] = sacc.y; g[2] = sacc.z; g[3] = sacc.w; }
     }
-    cl.sync();                               // nobody leaves while a peer may still read its tile
+    cl.sync();                               // nobody leaves while a peer may still read its block
 }
 
 // ------------------------------------------------------------------------------------------- C ABI
@@ -796,6 +834,22 @@ static int tile_plan(int B, int F, int R, int E, int mode, int* nstage_out, size
         return tm;
     }
     return 0;
+}
+
+// k_wgrad's launch: S batch slices (= cluster size) of >= 64 targets, and the output block width W. 64 x 64 blocks
+// when their clusters already cover the SMs (C3: 40 blocks x 8 slices); otherwise 32 x 32 blocks (C2: 7 -> 26 blocks
+// x 8 slices), which cut each CTA's fmaf chains to a quarter and let a C2-sized slice load behind a single wait.
+// Smaller blocks read more shared memory per FMA, so they are used only where they buy parallelism.
+struct WgradPlan { int S, W, clusters; };
+static WgradPlan wgrad_plan(int B, int F, int R, int E) {
+    WgradPlan w;
+    w.S = 8;
+    while (w.S > 1 && (B + w.S - 1) / w.S < 64) w.S >>= 1;
+    const int Fp = (F + 3) & ~3, K2p = Fp + R * E;
+    auto blocks = [&](int W) { return ((K2p + W - 1) / W + R * ((2 * Fp + W - 1) / W)) * ((E + W - 1) / W); };
+    w.W = blocks(64) * w.S >= pcg_device_sms() ? 64 : 32;
+    w.clusters = 1 + blocks(w.W);            // + the small-gradient cluster
+    return w;
 }
 
 extern "C" int pcg_tile_supported(int B, int R, int F, int E) {
@@ -918,26 +972,24 @@ extern "C" int pcg_tile_train(const float* feat, int64_t ldf, int F, const int32
     WgP w = {};
     w.cat = p.cat; w.ldcat = K2p; w.agg = agg; w.lda = lda; w.rep = agg_rep; w.dz = p.dz; w.dh = p.dh;
     w.B = B; w.F = F; w.Fp = Fp; w.R = R; w.E = E;
-    int S = 8;                               // batch slices = cluster size: slices of >= 64 targets
-    while (S > 1 && (B + S - 1) / S < 64) S >>= 1;
-    w.S = S;
+    const WgradPlan wp = wgrad_plan(B, F, R, E);
+    w.S = wp.S;
     w.grad[0] = d_w_inter;
     for (int j = 1; j <= R; ++j) w.grad[j] = d_w_intra_host[j - 1];
     w.partial = p.partial; w.n_tiles = (B + tm - 1) / tm; w.PS = tile_ps(F, E);
     w.lambda = lambda; w.loss = loss; w.d_w_head = d_w_head; w.d_w_clf = d_w_clf; w.d_b_clf = d_b_clf;
-    const int Mw = K2p > 2 * Fp ? K2p : 2 * Fp;
     cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)((Mw + 63) / 64), (unsigned)((E + 63) / 64), (unsigned)((R + 2) * S));
+    cfg.gridDim = dim3((unsigned)(wp.clusters * wp.S));
     cfg.blockDim = dim3(256);
     cfg.stream = stream;
     cudaLaunchAttribute attr[2];
     attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 1; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = (unsigned)S;
+    attr[0].val.clusterDim.x = (unsigned)wp.S; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
     attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[1].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
     cfg.numAttrs = (mask & 4) ? 2 : 1;
-    e = cudaLaunchKernelEx(&cfg, k_wgrad, w);
+    e = wp.W == 64 ? cudaLaunchKernelEx(&cfg, k_wgrad<64>, w) : cudaLaunchKernelEx(&cfg, k_wgrad<32>, w);
     if (e != cudaSuccess) { pcg_set_error("pcg_tile_train: wgrad launch: %s", cudaGetErrorString(e)); return (int)e; }
     return pcg_check_launch("pcg_tile_train");
 }
