@@ -389,10 +389,26 @@ PCG_API int pcg_score_bcast(const float* feat_rows, int64_t n_rows, int F, int64
  * statistic with average ranks for ties (NaN when one class is absent), the confusion counts take pred = 1 iff
  * prob[1] > prob[0], F1 / recall / precision follow sklearn's zero_division=0, and the best threshold is the distinct
  * value t of prob[1] whose cut "positive iff prob[1] >= t" has the largest macro-F1 (ties: the larger t).
- * Deterministic (integer sums, an order-free arg-max); 0 < n < 2^31.
+ * Ranking words, with s = prob[1] sorted ascending, P positives, N = n - P, pre[j] = positives among s[0, j)
+ * (pre[n] = P), a tie group = a maximal run [lo, hi) of equal s and its cut "positive iff prob[1] >= s[lo]"
+ * (TP = P - pre[lo], FP = (n - lo) - TP):
+ *   PCG_MT_AP           sklearn's average_precision_score: sum over groups of (pre[hi]-pre[lo])/P * TP/(n-lo); NaN if P = 0
+ *   PCG_MT_RECALL_AT_K  K = P: with c = n - P and [lo, hi) the group containing c,
+ *                       TP@K = (P - pre[hi]) + (pre[hi]-pre[lo]) * (hi-c)/(hi-lo) (the expected count over random
+ *                       orders of the tied scores), then / P; NaN if P = 0. With K = P it is also Precision@K.
+ *   PCG_MT_BEST_GMEAN   sqrt(TP/P * TN/N) maximised over the group cuts (0 where a denominator is 0), ties to the larger
+ *                       threshold; PCG_MT_BEST_GMEAN_THRESHOLD is that s[lo]
+ * Deterministic (integer sums, fp64 sums in a fixed order, an order-free arg-max); 0 < n < 2^31.
  *   workspace  pcg_binary_metrics_workspace_bytes(n) bytes, 256-byte aligned
+ * Words 17-20 were appended in version 101 (PCG_METRICS_WORDS was 17); words 0-16 are unchanged, so a caller that
+ * sizes `out` with PCG_METRICS_WORDS only needs to recompile.
+ *
+ * pcg_binary_curve: the ROC / PR curve of the last pcg_binary_metrics call on `workspace` (same n, ordered after it on
+ * the stream), read from the sorted scores and pre that call left there (no further sort). For the G tie groups in
+ * ascending order of threshold it writes thr[g] = s[lo], tp[g] = TP, fp[g] = FP of the group's cut, and G into the
+ * device word *count. thr, tp and fp must hold n entries (G <= n).
  */
-#define PCG_METRICS_WORDS 17
+#define PCG_METRICS_WORDS 21
 #define PCG_MT_AUC 0
 #define PCG_MT_F1 1
 #define PCG_MT_F1_MACRO 2
@@ -410,11 +426,17 @@ PCG_API int pcg_score_bcast(const float* feat_rows, int64_t n_rows, int F, int64
 #define PCG_MT_FP 14
 #define PCG_MT_TN 15
 #define PCG_MT_FN 16
+#define PCG_MT_AP 17
+#define PCG_MT_RECALL_AT_K 18
+#define PCG_MT_BEST_GMEAN 19
+#define PCG_MT_BEST_GMEAN_THRESHOLD 20
 PCG_API int pcg_eval_head(const float* emb, int E, int B, const float* w_head, int mode, int64_t n_total,
                   const uint32_t* cursor, uint32_t count, float* prob, pcg_stream_t stream);
 PCG_API size_t pcg_binary_metrics_workspace_bytes(int64_t n);
 PCG_API int pcg_binary_metrics(const float* prob, const int32_t* labels, int64_t n, double* out, void* workspace,
                        size_t workspace_bytes, pcg_stream_t stream);
+PCG_API int pcg_binary_curve(const void* workspace, size_t workspace_bytes, int64_t n, float* thr, int64_t* tp,
+                     int64_t* fp, int64_t* count, pcg_stream_t stream);
 
 #ifdef __cplusplus
 }

@@ -21,7 +21,8 @@ NORM_MEAN, NORM_RSQRT = 0, 1
 KB_MAX_POOL = 8192   # PCG_KB_WORDS * 32: pools up to this size use the per-item kept-pool bitmap
 # PCG_METRICS_WORDS doubles written by pcg_binary_metrics, in the order of the PCG_MT_* word indices
 METRICS_KEYS = ("auc", "f1", "f1_macro", "recall", "precision", "recall_macro", "precision_macro", "accuracy", "gmean",
-                "best_f1_macro", "best_threshold", "n_pos", "n_neg", "tp", "fp", "tn", "fn")
+                "best_f1_macro", "best_threshold", "n_pos", "n_neg", "tp", "fp", "tn", "fn",
+                "ap", "recall_at_k", "best_gmean", "best_gmean_threshold")
 METRICS_WORDS = len(METRICS_KEYS)
 
 _p = C.c_void_p
@@ -86,6 +87,7 @@ SIGNATURES = {
     "pcg_eval_head": (_i, [_p, _i, _i, _p, _i, _l, _p, C.c_uint32, _p, _p]),
     "pcg_binary_metrics_workspace_bytes": (_z, [_l]),
     "pcg_binary_metrics": (_i, [_p, _p, _l, _p, _p, _z, _p]),
+    "pcg_binary_curve": (_i, [_p, _z, _l, _p, _p, _p, _p, _p]),
 }
 
 _lib = None

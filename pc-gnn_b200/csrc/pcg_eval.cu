@@ -1,7 +1,8 @@
 // Evaluation pass on the device: the two-class head + sigmoid (PCALayer, GCN) or log-softmax (GraphSage) into a
 // whole-set probability buffer, and the binary metrics of src/utils.py:298-333 (AUC, F1, recall, precision, ...) plus
-// a best-threshold macro-F1, computed where the probabilities live. Deterministic: integer sums and an order-free
-// arg-max only (no floating-point atomics).
+// the ranking metrics of fraud-detection benchmarks (average precision, Recall@K, the best macro-F1 and G-mean cuts)
+// and the ROC / PR curve, computed where the probabilities live. Deterministic: integer sums, fp64 sums in a fixed
+// order and an order-free arg-max only (no floating-point atomics).
 #include <math.h>
 
 #include "pcg_common.cuh"
@@ -55,8 +56,26 @@ extern "C" int pcg_eval_head(const float* emb, int E, int B, const float* w_head
 //                    lower / upper bound: twice the average rank = lo + hi + 1), and the confusion counts of the
 //                    chunk's ORIGINAL positions (pred = prob[1] > prob[0], the argmax of utils.test)
 //   k_metrics_best   per chunk: positives in front of every position (chunk prefix from the counts + a block scan),
-//                    macro-F1 of the cut "positive iff prob[1] >= s[j]" at every tie-group start j, the chunk's best
-//   k_metrics_final  one CTA: sums and arg-max over the chunks, every metric in double
+//                    stored as pre[j]; macro-F1 and G-mean of the cut "positive iff prob[1] >= s[j]" at every tie-group
+//                    start j, the chunk's best of each, and the number of group starts in the chunk
+//   k_metrics_ap     per chunk, once pre is complete: the chunk's positives' average-precision terms, summed in fp64
+//   k_metrics_final  one CTA: sums and arg-max over the chunks, Recall@K, every metric in double
+// pcg_binary_curve reads the sorted scores and pre back: k_curve_scan (one CTA) is an exclusive scan of the chunks'
+// group-start counts, k_curve_write writes each chunk's groups at that offset (block scan inside the chunk).
+//
+// Definitions (s = prob[1] sorted ascending, n nodes, P positives, N = n - P):
+//   pre[j]      positives among s[0, j); pre[n] = P
+//   tie group   a maximal run [lo, hi) of equal s; its cut is "positive iff prob[1] >= s[lo]", so
+//               TP = P - pre[lo], FP = (n - lo) - TP
+//   ap          sklearn's average_precision_score: sum over groups of (pre[hi] - pre[lo]) / P * TP / (n - lo). Every
+//               positive of a group carries the group's precision, so this is summed as (1/P) * sum over positives of
+//               TP / (n - lo) with lo = lower_bound(s, s[j]) (no group end needed). NaN when P = 0.
+//   recall_at_k K = P alerts: with c = n - P and [lo, hi) the group that contains position c,
+//               TP@K = (P - pre[hi]) + (pre[hi] - pre[lo]) * (hi - c) / (hi - lo), the expected count over random
+//               orders of the tied scores (independent of the sort's tie order), then / P. NaN when P = 0. Since K = P
+//               it is Precision@K as well.
+//   best_gmean  sqrt(TP/P * TN/N) maximised over the group cuts (a ratio with a zero denominator is 0), ties to the
+//               larger threshold, as best_f1_macro
 #define MT_NT 256
 #define MT_PER 8
 #define MT_CH (MT_NT * MT_PER)
@@ -68,6 +87,11 @@ struct MetricsBlk {
 struct BestBlk {
     double f1;
     long long at;          // sorted position of the cut (-1: none in this chunk)
+    double gm;             // best G-mean and its cut
+    long long gat;
+    double ap;             // sum over the chunk's positives of TP / (n - lo) (k_metrics_ap)
+    long long groups;      // tie-group starts in the chunk
+    long long goff;        // group starts in front of the chunk (k_curve_scan)
 };
 
 static size_t align256(size_t x) { return (x + 255) & ~(size_t)255; }
@@ -80,6 +104,7 @@ struct MetricsWs {
     int32_t* s_lab;
     MetricsBlk* blk;
     BestBlk* best;
+    int32_t* pre;
     size_t total;
 };
 
@@ -94,6 +119,7 @@ static MetricsWs metrics_layout(char* base, int64_t n) {
     w.s_lab = (int32_t*)(base + o);   o += align256((size_t)n * 4);
     w.blk = (MetricsBlk*)(base + o);  o += align256((size_t)nb * sizeof(MetricsBlk));
     w.best = (BestBlk*)(base + o);    o += align256((size_t)nb * sizeof(BestBlk));
+    w.pre = (int32_t*)(base + o);     o += align256((size_t)n * 4);
     w.total = o;
     return w;
 }
@@ -172,16 +198,43 @@ __device__ __forceinline__ bool better(double f, long long at, double bf, long l
     return f > bf || (f == bf && at > bat);      // ties: the larger threshold
 }
 
+// (bf, bat) <- the better() maximum over the warp, in every lane
+__device__ __forceinline__ void argmax_warp(double& bf, long long& bat) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        const double of = __shfl_xor_sync(PCG_FULL, bf, o);
+        const long long oat = __shfl_xor_sync(PCG_FULL, bat, o);
+        if (better(of, oat, bf, bat)) { bf = of; bat = oat; }
+    }
+}
+
+// exclusive prefix sum of v over the CTA's threads in thread order; warp_tot: MT_NT / 32 ints of shared memory, one
+// call per kernel
+__device__ __forceinline__ int block_excl_scan(int v, int* warp_tot) {
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    int incl = v;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const int y = __shfl_up_sync(PCG_FULL, incl, o);
+        if (lane >= o) incl += y;
+    }
+    if (lane == 31) warp_tot[wid] = incl;
+    __syncthreads();
+    int run = incl - v;
+    for (int q = 0; q < wid; ++q) run += warp_tot[q];
+    return run;
+}
+
 __global__ void __launch_bounds__(MT_NT) k_metrics_best(int64_t n, const float* __restrict__ s_score,
                                                         const int32_t* __restrict__ s_lab,
                                                         const MetricsBlk* __restrict__ blk, int nb,
-                                                        BestBlk* __restrict__ best) {
+                                                        BestBlk* __restrict__ best, int32_t* __restrict__ pre) {
     __shared__ long long red[MT_NT / 32];
     __shared__ int lab_s[MT_CH];
     __shared__ float sc_s[MT_CH + 1];
     __shared__ int warp_tot[MT_NT / 32];
-    __shared__ double bf_s[MT_NT / 32];
-    __shared__ long long bat_s[MT_NT / 32];
+    __shared__ double bf_s[MT_NT / 32], bg_s[MT_NT / 32];
+    __shared__ long long bat_s[MT_NT / 32], bgat_s[MT_NT / 32];
     __shared__ long long pos_all, pos_before;
     const int64_t j0 = (int64_t)blockIdx.x * MT_CH;
     // positives over all chunks and in front of this one
@@ -206,78 +259,101 @@ __global__ void __launch_bounds__(MT_NT) k_metrics_best(int64_t n, const float* 
     int mine = 0;
 #pragma unroll
     for (int u = 0; u < MT_PER; ++u) mine += lab_s[threadIdx.x * MT_PER + u];
+    const int run = block_excl_scan(mine, warp_tot);
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    int incl = mine;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        const int y = __shfl_up_sync(PCG_FULL, incl, o);
-        if (lane >= o) incl += y;
-    }
-    if (lane == 31) warp_tot[wid] = incl;
-    __syncthreads();
-    int run = incl - mine;
-    for (int q = 0; q < wid; ++q) run += warp_tot[q];
     const double P = (double)pos_all, N = (double)(n - pos_all);
     long long cnt = pos_before + run;          // positives in front of the current position
-    double bf = -1.0;
-    long long bat = -1;
+    double bf = -1.0, bg = -1.0;
+    long long bat = -1, bgat = -1, groups = 0;
     for (int u = 0; u < MT_PER; ++u) {
         const int k = threadIdx.x * MT_PER + u;
         const int64_t j = j0 + k;
         if (j >= n) break;
+        pre[j] = (int32_t)cnt;
         if (j == 0 || sc_s[k + 1] != sc_s[k]) {
             const double tp = P - (double)cnt, pp = (double)(n - j);
             const double fp = pp - tp, fn = P - tp, tn = N - fp;
             const double f = f1_pair(tp, fp, tn, fn, nullptr);
             if (better(f, j, bf, bat)) { bf = f; bat = j; }
+            const double g = sqrt(__dmul_rn(ratio(tp, P), ratio(tn, N)));
+            if (better(g, j, bg, bgat)) { bg = g; bgat = j; }
+            ++groups;
         }
         cnt += lab_s[k];
     }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-        const double of = __shfl_xor_sync(PCG_FULL, bf, o);
-        const long long oat = __shfl_xor_sync(PCG_FULL, bat, o);
-        if (better(of, oat, bf, bat)) { bf = of; bat = oat; }
-    }
-    if (lane == 0) { bf_s[wid] = bf; bat_s[wid] = bat; }
+    groups = block_sum(groups, red);
+    argmax_warp(bf, bat);
+    argmax_warp(bg, bgat);
+    if (lane == 0) { bf_s[wid] = bf; bat_s[wid] = bat; bg_s[wid] = bg; bgat_s[wid] = bgat; }
     __syncthreads();
     if (threadIdx.x == 0) {
-        for (int q = 1; q < MT_NT / 32; ++q)
+        for (int q = 1; q < MT_NT / 32; ++q) {
             if (better(bf_s[q], bat_s[q], bf, bat)) { bf = bf_s[q]; bat = bat_s[q]; }
-        best[blockIdx.x].f1 = bf;
-        best[blockIdx.x].at = bat;
+            if (better(bg_s[q], bgat_s[q], bg, bgat)) { bg = bg_s[q]; bgat = bgat_s[q]; }
+        }
+        BestBlk& b = best[blockIdx.x];
+        b.f1 = bf;
+        b.at = bat;
+        b.gm = bg;
+        b.gat = bgat;
+        b.groups = groups;
     }
 }
 
+// Average-precision terms of the chunk's positives (see the definitions above): sum of TP / (n - lo) over the
+// positives at sorted positions j of the chunk, lo = the start of j's tie group. Needs pre of every chunk.
+__global__ void __launch_bounds__(MT_NT) k_metrics_ap(int64_t n, const float* __restrict__ s_score,
+                                                      const int32_t* __restrict__ s_lab, const int32_t* __restrict__ pre,
+                                                      BestBlk* __restrict__ best) {
+    __shared__ double red[MT_NT / 32];
+    const int64_t j0 = (int64_t)blockIdx.x * MT_CH;
+    const long long P = (long long)pre[n - 1] + (s_lab[n - 1] != 0);
+    double acc = 0.0;
+    for (int u = 0; u < MT_PER; ++u) {
+        const int64_t j = j0 + u * MT_NT + threadIdx.x;
+        if (j >= n) break;
+        if (s_lab[j] != 0) {
+            const int64_t lo = bound(s_score, n, s_score[j], false);
+            acc += (double)(P - pre[lo]) / (double)(n - lo);
+        }
+    }
+    acc = block_sum(acc, red);
+    if (threadIdx.x == 0) best[blockIdx.x].ap = acc;
+}
+
 __global__ void __launch_bounds__(MT_NT) k_metrics_final(int64_t n, const float* __restrict__ s_score,
+                                                         const int32_t* __restrict__ pre,
                                                          const MetricsBlk* __restrict__ blk, const BestBlk* __restrict__ best,
                                                          int nb, double* __restrict__ out) {
     __shared__ long long red[MT_NT / 32];
-    __shared__ double bf_s[MT_NT / 32];
-    __shared__ long long bat_s[MT_NT / 32];
+    __shared__ double red_d[MT_NT / 32];
+    __shared__ double bf_s[MT_NT / 32], bg_s[MT_NT / 32];
+    __shared__ long long bat_s[MT_NT / 32], bgat_s[MT_NT / 32];
     long long c[6] = {0, 0, 0, 0, 0, 0};       // auc2, pos, tp, fp, tn, fn
-    double bf = -1.0;
-    long long bat = -1;
+    double bf = -1.0, bg = -1.0, ap = 0.0;
+    long long bat = -1, bgat = -1;
     for (int b = threadIdx.x; b < nb; b += MT_NT) {
         const MetricsBlk m = blk[b];
         c[0] += m.auc2; c[1] += m.pos; c[2] += m.tp; c[3] += m.fp; c[4] += m.tn; c[5] += m.fn;
-        if (better(best[b].f1, best[b].at, bf, bat)) { bf = best[b].f1; bat = best[b].at; }
+        const BestBlk k = best[b];
+        if (better(k.f1, k.at, bf, bat)) { bf = k.f1; bat = k.at; }
+        if (better(k.gm, k.gat, bg, bgat)) { bg = k.gm; bgat = k.gat; }
+        ap += k.ap;                           // chunks b, b + MT_NT, ... in order, then a fixed tree: same bits on reruns
     }
     long long t[6];
 #pragma unroll
     for (int q = 0; q < 6; ++q) t[q] = block_sum(c[q], red);
+    ap = block_sum(ap, red_d);
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-        const double of = __shfl_xor_sync(PCG_FULL, bf, o);
-        const long long oat = __shfl_xor_sync(PCG_FULL, bat, o);
-        if (better(of, oat, bf, bat)) { bf = of; bat = oat; }
-    }
-    if (lane == 0) { bf_s[wid] = bf; bat_s[wid] = bat; }
+    argmax_warp(bf, bat);
+    argmax_warp(bg, bgat);
+    if (lane == 0) { bf_s[wid] = bf; bat_s[wid] = bat; bg_s[wid] = bg; bgat_s[wid] = bgat; }
     __syncthreads();
     if (threadIdx.x != 0) return;
-    for (int q = 1; q < MT_NT / 32; ++q)
+    for (int q = 1; q < MT_NT / 32; ++q) {
         if (better(bf_s[q], bat_s[q], bf, bat)) { bf = bf_s[q]; bat = bat_s[q]; }
+        if (better(bg_s[q], bgat_s[q], bg, bgat)) { bg = bg_s[q]; bgat = bgat_s[q]; }
+    }
     const long long P = t[1], N = n - t[1];
     const double tp = (double)t[2], fp = (double)t[3], tn = (double)t[4], fn = (double)t[5];
     // Mann-Whitney U with average ranks: 2U = sum_pos (lo + hi + 1) - P(P+1), exact in int64
@@ -300,6 +376,75 @@ __global__ void __launch_bounds__(MT_NT) k_metrics_final(int64_t n, const float*
     out[PCG_MT_FP] = fp;
     out[PCG_MT_TN] = tn;
     out[PCG_MT_FN] = fn;
+    out[PCG_MT_AP] = P > 0 ? ap / (double)P : nan("");
+    double rk = nan("");
+    if (P > 0) {                               // K = P: the top P positions are c .. n-1
+        const int64_t c_ = n - P;
+        const float x = s_score[c_];
+        const int64_t lo = bound(s_score, n, x, false), hi = bound(s_score, n, x, true);
+        const long long plo = pre[lo], phi = hi < n ? (long long)pre[hi] : P;
+        const double tpk = (double)(P - phi) + (double)(phi - plo) * (double)(hi - c_) / (double)(hi - lo);
+        rk = tpk / (double)P;
+    }
+    out[PCG_MT_RECALL_AT_K] = rk;
+    out[PCG_MT_BEST_GMEAN] = bg;
+    out[PCG_MT_BEST_GMEAN_THRESHOLD] = (double)s_score[bgat];
+}
+
+// Exclusive scan of the chunks' group-start counts into best[b].goff (one CTA, MT_NT chunks per round); *count = G.
+__global__ void __launch_bounds__(MT_NT) k_curve_scan(BestBlk* __restrict__ best, int nb, int64_t* __restrict__ count) {
+    __shared__ int warp_tot[MT_NT / 32];
+    __shared__ long long carry;
+    if (threadIdx.x == 0) carry = 0;
+    for (int b0 = 0; b0 < nb; b0 += MT_NT) {
+        const int b = b0 + threadIdx.x;
+        const int g = b < nb ? (int)best[b].groups : 0;
+        __syncthreads();                       // carry written, warp_tot free for the next round
+        const int run = block_excl_scan(g, warp_tot);
+        if (b < nb) best[b].goff = carry + run;
+        __syncthreads();
+        if (threadIdx.x == MT_NT - 1) carry += run + g;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) *count = carry;
+}
+
+// Each chunk's group starts j, in order, at best[chunk].goff: thr = s[j], tp = P - pre[j], fp = (n - j) - tp.
+__global__ void __launch_bounds__(MT_NT) k_curve_write(int64_t n, const float* __restrict__ s_score,
+                                                       const int32_t* __restrict__ s_lab, const int32_t* __restrict__ pre,
+                                                       const BestBlk* __restrict__ best, float* __restrict__ thr,
+                                                       int64_t* __restrict__ tp, int64_t* __restrict__ fp) {
+    __shared__ float sc_s[MT_CH + 1];
+    __shared__ int warp_tot[MT_NT / 32];
+    const int64_t j0 = (int64_t)blockIdx.x * MT_CH;
+    for (int u = 0; u < MT_PER; ++u) {
+        const int k = u * MT_NT + threadIdx.x;
+        const int64_t j = j0 + k;
+        sc_s[k + 1] = j < n ? s_score[j] : 0.f;
+    }
+    if (threadIdx.x == 0) sc_s[0] = j0 > 0 ? s_score[j0 - 1] : 0.f;
+    __syncthreads();
+    const long long P = (long long)pre[n - 1] + (s_lab[n - 1] != 0);
+    int mine = 0;
+#pragma unroll
+    for (int u = 0; u < MT_PER; ++u) {
+        const int k = threadIdx.x * MT_PER + u;
+        const int64_t j = j0 + k;
+        mine += j < n && (j == 0 || sc_s[k + 1] != sc_s[k]);
+    }
+    long long at = best[blockIdx.x].goff + block_excl_scan(mine, warp_tot);
+    for (int u = 0; u < MT_PER; ++u) {
+        const int k = threadIdx.x * MT_PER + u;
+        const int64_t j = j0 + k;
+        if (j >= n) break;
+        if (j == 0 || sc_s[k + 1] != sc_s[k]) {
+            const long long t = P - pre[j];
+            thr[at] = sc_s[k + 1];
+            tp[at] = t;
+            fp[at] = (n - j) - t;
+            ++at;
+        }
+    }
 }
 
 extern "C" size_t pcg_binary_metrics_workspace_bytes(int64_t n) {
@@ -319,7 +464,22 @@ extern "C" int pcg_binary_metrics(const float* prob, const int32_t* labels, int6
     int rc = pcg_sort_pool(prob + n, labels, (int)n, w.s_score, w.s_pos, w.s_lab, w.sort_ws, w.sort_bytes, stream_);
     if (rc) return rc;
     k_metrics_count<<<nb, MT_NT, 0, stream>>>(prob, labels, n, w.s_score, w.s_lab, w.blk);
-    k_metrics_best<<<nb, MT_NT, 0, stream>>>(n, w.s_score, w.s_lab, w.blk, nb, w.best);
-    k_metrics_final<<<1, MT_NT, 0, stream>>>(n, w.s_score, w.blk, w.best, nb, out);
+    k_metrics_best<<<nb, MT_NT, 0, stream>>>(n, w.s_score, w.s_lab, w.blk, nb, w.best, w.pre);
+    k_metrics_ap<<<nb, MT_NT, 0, stream>>>(n, w.s_score, w.s_lab, w.pre, w.best);
+    k_metrics_final<<<1, MT_NT, 0, stream>>>(n, w.s_score, w.pre, w.blk, w.best, nb, out);
     return pcg_check_launch("pcg_binary_metrics");
+}
+
+extern "C" int pcg_binary_curve(const void* workspace, size_t workspace_bytes, int64_t n, float* thr, int64_t* tp,
+                                int64_t* fp, int64_t* count, pcg_stream_t stream_) {
+    cudaStream_t stream = (cudaStream_t)stream_;
+    PCG_REQUIRE(workspace && thr && tp && fp && count, "pcg_binary_curve: null pointer");
+    PCG_REQUIRE(n > 0 && n <= 0x7fffffff, "pcg_binary_curve: need 0 < n < 2^31 (n=%lld)", (long long)n);
+    const MetricsWs w = metrics_layout((char*)workspace, n);
+    PCG_REQUIRE(((uintptr_t)workspace & 255) == 0 && workspace_bytes >= w.total,
+                "pcg_binary_curve: workspace must be 256-byte aligned and pcg_binary_metrics_workspace_bytes(n) long");
+    const int nb = (int)((n + MT_CH - 1) / MT_CH);
+    k_curve_scan<<<1, MT_NT, 0, stream>>>(w.best, nb, count);
+    k_curve_write<<<nb, MT_NT, 0, stream>>>(n, w.s_score, w.s_lab, w.pre, w.best, thr, tp, fp);
+    return pcg_check_launch("pcg_binary_curve");
 }

@@ -12,7 +12,7 @@ from __future__ import annotations
 
 import torch
 
-__all__ = ["binary_metrics", "device_metrics"]
+__all__ = ["binary_metrics", "device_metrics", "device_curve"]
 
 
 def binary_metrics(prob1: torch.Tensor, pred: torch.Tensor, labels: torch.Tensor) -> dict:
@@ -52,29 +52,68 @@ def binary_metrics(prob1: torch.Tensor, pred: torch.Tensor, labels: torch.Tensor
     return dict(zip(keys, out))
 
 
-def device_metrics(prob_2n: torch.Tensor, labels: torch.Tensor) -> dict:
-    """``binary_metrics`` of pred = (prob[1] > prob[0]) computed by one kernel chain (``pcg_binary_metrics``: sort,
-    counts, best threshold) plus one device->host copy. prob_2n: planar [2, n] fp32 CUDA tensor (row 1 = P(class 1));
-    labels: 0 / 1 per node. Returns python floats: the keys of ``binary_metrics`` plus best_f1_macro / best_threshold
-    (the distinct value t of prob[1] whose cut "positive iff prob[1] >= t" has the largest macro-F1, ties to the larger
-    t), n_pos, n_neg and the confusion counts tp, fp, tn, fn."""
+def _run_metrics(prob_2n, labels, what):
+    """pcg_binary_metrics on a fresh workspace: (n, workspace, out) on the probabilities' device."""
     from . import _lib
 
     if prob_2n.dim() != 2 or prob_2n.shape[0] != 2 or not prob_2n.is_cuda:
-        raise ValueError(f"device_metrics: prob must be a [2, n] CUDA tensor, got {tuple(prob_2n.shape)}")
+        raise ValueError(f"{what}: prob must be a [2, n] CUDA tensor, got {tuple(prob_2n.shape)}")
     n = int(prob_2n.shape[1])
     if n == 0:
-        raise ValueError("device_metrics: no nodes")
+        raise ValueError(f"{what}: no nodes")
     prob = prob_2n.to(torch.float32).contiguous()
     y = torch.as_tensor(labels, device=prob.device).reshape(-1)
     if y.numel() != n:
-        raise ValueError(f"device_metrics: {y.numel()} labels for {n} nodes")
+        raise ValueError(f"{what}: {y.numel()} labels for {n} nodes")
     if bool(((y != 0) & (y != 1)).any()):
-        raise ValueError("device_metrics: labels must be 0 or 1")
+        raise ValueError(f"{what}: labels must be 0 or 1")
     y = y.to(torch.int32).contiguous()
     L = _lib.lib()
     ws = torch.empty(int(L.pcg_binary_metrics_workspace_bytes(n)), dtype=torch.uint8, device=prob.device)
     out = torch.empty(_lib.METRICS_WORDS, dtype=torch.float64, device=prob.device)
     _lib.check(L.pcg_binary_metrics(prob.data_ptr(), y.data_ptr(), n, out.data_ptr(), ws.data_ptr(), ws.numel(),
                                     _lib.stream_ptr()), "pcg_binary_metrics")
+    return n, ws, out
+
+
+def device_metrics(prob_2n: torch.Tensor, labels: torch.Tensor) -> dict:
+    """``binary_metrics`` of pred = (prob[1] > prob[0]) computed by one kernel chain (``pcg_binary_metrics``: sort,
+    counts, best threshold) plus one device->host copy. prob_2n: planar [2, n] fp32 CUDA tensor (row 1 = P(class 1));
+    labels: 0 / 1 per node. Returns python floats: the keys of ``binary_metrics`` plus best_f1_macro / best_threshold
+    (the distinct value t of prob[1] whose cut "positive iff prob[1] >= t" has the largest macro-F1, ties to the larger
+    t), n_pos, n_neg, the confusion counts tp, fp, tn, fn, and the ranking metrics: ap (sklearn's
+    average_precision_score), recall_at_k (K = n_pos, ties counted by their expected share; also Precision@K) and
+    best_gmean / best_gmean_threshold (the cut with the largest sqrt(TPR * TNR), ties to the larger t). ap and
+    recall_at_k are NaN without positives. Definitions: include/pcgnn_b200.h."""
+    from . import _lib
+
+    _, _, out = _run_metrics(prob_2n, labels, "device_metrics")
     return dict(zip(_lib.METRICS_KEYS, out.cpu().tolist()))
+
+
+def _curve_buffers(n: int, device):
+    """(thr fp32 [n], tp int64 [n], fp int64 [n], count int64 [1]): the outputs of ``pcg_binary_curve``."""
+    return (torch.empty(n, dtype=torch.float32, device=device), torch.empty(n, dtype=torch.int64, device=device),
+            torch.empty(n, dtype=torch.int64, device=device), torch.empty(1, dtype=torch.int64, device=device))
+
+
+def _read_curve(ws: torch.Tensor, n: int, bufs) -> tuple:
+    """``pcg_binary_curve`` over a workspace the last ``pcg_binary_metrics`` on the current stream filled, then one
+    8-byte read of G: views [:G] of the buffers."""
+    from . import _lib
+
+    thr, tp, fp, count = bufs
+    _lib.check(_lib.lib().pcg_binary_curve(ws.data_ptr(), ws.numel(), n, thr.data_ptr(), tp.data_ptr(), fp.data_ptr(),
+                                           count.data_ptr(), _lib.stream_ptr()), "pcg_binary_curve")
+    G = int(count.item())
+    return thr[:G], tp[:G], fp[:G]
+
+
+def device_curve(prob_2n: torch.Tensor, labels: torch.Tensor) -> tuple:
+    """ROC / PR curve of prob[1] against 0 / 1 labels: (thresholds fp32 [G], tp int64 [G], fp int64 [G]) as device
+    tensors, one entry per distinct value t of prob[1] in ascending order with the counts of the cut "positive iff
+    prob[1] >= t". TPR = tp / n_pos, FPR = fp / n_neg, precision = tp / (tp + fp): sklearn's roc_curve
+    (drop_intermediate=False) and precision_recall_curve in reverse order, without their sentinel point.
+    ``pcg_binary_metrics`` (sort) then ``pcg_binary_curve`` (no further sort) and one 8-byte read of G."""
+    n, ws, _ = _run_metrics(prob_2n, labels, "device_curve")
+    return _read_curve(ws, n, _curve_buffers(n, prob_2n.device))

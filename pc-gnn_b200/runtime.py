@@ -499,6 +499,8 @@ class GraphedEvalPass:
             self.cap_slots = self._baseline_capacity()
         self._done = torch.cuda.Event()
         self._key = None
+        self._curve = None                             # pcg_binary_curve's outputs, allocated by the first curve()
+        self._ran = False
         self.g_batch = self.g_metrics = None
         self.captures = 0
 
@@ -638,9 +640,11 @@ class GraphedEvalPass:
 
     def run(self) -> dict:
         """Scores every node and returns the metrics as python floats: the keys of ``metrics.binary_metrics`` (pred =
-        prob[1] > prob[0], as utils.test) plus best_f1_macro, best_threshold, n_pos, n_neg and tp / fp / tn / fn.
+        prob[1] > prob[0], as utils.test) plus best_f1_macro, best_threshold, n_pos, n_neg, tp / fp / tn / fn, ap,
+        recall_at_k, best_gmean and best_gmean_threshold (``metrics.device_metrics``).
         The metrics are computed on ``probs()`` as they are: for GraphSage, log-probabilities, so ``best_threshold``
-        is a log-probability there (pred and AUC are unchanged by the log).
+        and ``best_gmean_threshold`` are log-probabilities there (pred, AUC and the ranking keys ap, recall_at_k,
+        best_f1_macro and best_gmean need no conversion: log is monotone).
         Raises PcgError when a batch needed more slots than ``cap_slots`` (its scores would be incomplete)."""
         key = self._state()
         if key != self._key:
@@ -651,6 +655,7 @@ class GraphedEvalPass:
         for _ in range(self.n_entries):
             self.g_batch.replay()
         self.g_metrics.replay()
+        self._ran = True
         self._done.record(torch.cuda.current_stream(self._prob.device))
         self._done.synchronize()
         W = _lib.METRICS_WORDS
@@ -659,6 +664,19 @@ class GraphedEvalPass:
             raise _lib.PcgError(f"GraphedEvalPass: {bad.size} of {self.n_entries} batches needed more than cap_slots="
                                 f"{self.cap_slots} slots (first: entry {int(bad[0])}); build the pass with a larger capacity")
         return dict(zip(_lib.METRICS_KEYS, self._pin_np[:2 * W].view(np.float64).tolist()))
+
+    def curve(self) -> tuple:
+        """ROC / PR curve of the last ``run()`` (``metrics.device_curve`` of ``probs()``): (thresholds fp32 [G],
+        tp int64 [G], fp int64 [G]) on the device, ascending thresholds. One eager launch over the metrics workspace
+        the run left and one 8-byte read of G; the tensors are views of buffers of the pass that the next ``curve()``
+        overwrites. For GraphSage the thresholds are log-probabilities (the counts are those of the probabilities)."""
+        from .metrics import _curve_buffers, _read_curve
+
+        if not self._ran:
+            raise _lib.PcgError("GraphedEvalPass.curve: run() first (the curve is read from the last run's metrics)")
+        if self._curve is None:
+            self._curve = _curve_buffers(self.n, self._prob.device)
+        return _read_curve(self._mws, self.n, self._curve)
 
     def probs(self) -> torch.Tensor:
         """[n, 2] view of the last run's to_prob output (PCALayer: its first output), in the caller's node order:
