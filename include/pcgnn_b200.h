@@ -407,6 +407,27 @@ PCG_API int pcg_score_bcast(const float* feat_rows, int64_t n_rows, int F, int64
  * the stream), read from the sorted scores and pre that call left there (no further sort). For the G tie groups in
  * ascending order of threshold it writes thr[g] = s[lo], tp[g] = TP, fp[g] = FP of the group's cut, and G into the
  * device word *count. thr, tp and fp must hold n entries (G <= n).
+ *
+ * pcg_binary_points: operating points the caller chooses, read like pcg_binary_curve from the workspace of the last
+ * pcg_binary_metrics call (same n, ordered after it on the stream; no further sort). Request r is kind[r] with the
+ * argument arg[r]; both arrays live in device memory, so a recorded graph keeps reading them and the caller may change
+ * them in place between replays. Request r writes out[r * PCG_POINT_WORDS + 0 .. 4]:
+ *   kind 0  top K (arg = K, an integer, 1 <= K <= n): with c = n - K and [lo, hi) the group containing c,
+ *           TP@K = (P - pre[hi]) + (pre[hi]-pre[lo]) * (hi-c)/(hi-lo) (PCG_MT_RECALL_AT_K's rule for any K).
+ *           Words {recall = TP@K / P (NaN if P = 0), precision = TP@K / K, threshold = s[c] (the K-th highest score),
+ *           TP@K, K - TP@K}. With K = P, recall has the bits of PCG_MT_RECALL_AT_K.
+ *   kind 1  TPR at FPR <= f (arg = f, 0 <= f <= 1): of the group cuts with FP(lo) <= f * N (compared in fp64) the one
+ *           with the largest TPR, i.e. the smallest such lo; when none has, nothing is flagged (TP = FP = 0, threshold
+ *           +inf). Words {TPR = TP / P, FPR = FP / N, threshold = s[lo], TP, FP}; all NaN if P = 0 or N = 0.
+ *   kind 2  standardised partial AUC (arg = max_fpr f, 0 < f <= 1), sklearn's roc_auc_score(max_fpr=f): A = the
+ *           trapezoid area under the ROC points (FP(lo)/N, TP(lo)/P) of the group starts and (0, 0), up to FPR = f
+ *           with TPR interpolated linearly at f. Words {0.5 * (1 + (A - f^2/2) / (f - f^2/2)), A, NaN, NaN, NaN};
+ *           with f = 1 the first is the AUC. NaN if P = 0 or N = 0.
+ * A request whose argument is out of its range, or whose kind is not 0, 1 or 2, writes PCG_POINT_WORDS NaN; words a
+ * kind does not define are NaN. Two launches whatever m is (0 < m <= PCG_POINTS_MAX); kind 2 sums fp64 partials per
+ * chunk in a fixed order, so reruns give the same bits.
+ *   metrics_ws  the workspace of pcg_binary_metrics (pcg_binary_metrics_workspace_bytes(n) bytes), not modified
+ *   ws          pcg_binary_points_workspace_bytes(n, m) bytes, 8-byte aligned (kind 2's partials)
  */
 #define PCG_METRICS_WORDS 21
 #define PCG_MT_AUC 0
@@ -430,6 +451,12 @@ PCG_API int pcg_score_bcast(const float* feat_rows, int64_t n_rows, int F, int64
 #define PCG_MT_RECALL_AT_K 18
 #define PCG_MT_BEST_GMEAN 19
 #define PCG_MT_BEST_GMEAN_THRESHOLD 20
+/* pcg_binary_points: doubles per request, most requests per call, request kinds */
+#define PCG_POINT_WORDS 5
+#define PCG_POINTS_MAX 1024
+#define PCG_POINT_TOP_K 0
+#define PCG_POINT_TPR_AT_FPR 1
+#define PCG_POINT_PAUC 2
 PCG_API int pcg_eval_head(const float* emb, int E, int B, const float* w_head, int mode, int64_t n_total,
                   const uint32_t* cursor, uint32_t count, float* prob, pcg_stream_t stream);
 PCG_API size_t pcg_binary_metrics_workspace_bytes(int64_t n);
@@ -437,6 +464,9 @@ PCG_API int pcg_binary_metrics(const float* prob, const int32_t* labels, int64_t
                        size_t workspace_bytes, pcg_stream_t stream);
 PCG_API int pcg_binary_curve(const void* workspace, size_t workspace_bytes, int64_t n, float* thr, int64_t* tp,
                      int64_t* fp, int64_t* count, pcg_stream_t stream);
+PCG_API size_t pcg_binary_points_workspace_bytes(int64_t n, int m);
+PCG_API int pcg_binary_points(const void* metrics_ws, size_t metrics_ws_bytes, int64_t n, const int32_t* kind,
+                      const double* arg, int m, double* out, void* ws, size_t ws_bytes, pcg_stream_t stream);
 
 #ifdef __cplusplus
 }

@@ -24,6 +24,9 @@ METRICS_KEYS = ("auc", "f1", "f1_macro", "recall", "precision", "recall_macro", 
                 "best_f1_macro", "best_threshold", "n_pos", "n_neg", "tp", "fp", "tn", "fn",
                 "ap", "recall_at_k", "best_gmean", "best_gmean_threshold")
 METRICS_WORDS = len(METRICS_KEYS)
+POINT_WORDS = 5      # PCG_POINT_WORDS: doubles per pcg_binary_points request
+POINTS_MAX = 1024    # PCG_POINTS_MAX
+POINT_TOP_K, POINT_TPR_AT_FPR, POINT_PAUC = 0, 1, 2
 
 _p = C.c_void_p
 _i = C.c_int
@@ -88,6 +91,8 @@ SIGNATURES = {
     "pcg_binary_metrics_workspace_bytes": (_z, [_l]),
     "pcg_binary_metrics": (_i, [_p, _p, _l, _p, _p, _z, _p]),
     "pcg_binary_curve": (_i, [_p, _z, _l, _p, _p, _p, _p, _p]),
+    "pcg_binary_points_workspace_bytes": (_z, [_l, _i]),
+    "pcg_binary_points": (_i, [_p, _z, _l, _p, _p, _i, _p, _p, _z, _p]),
 }
 
 _lib = None

@@ -321,6 +321,19 @@ __global__ void __launch_bounds__(MT_NT) k_metrics_ap(int64_t n, const float* __
     if (threadIdx.x == 0) best[blockIdx.x].ap = acc;
 }
 
+// TP@K of the top K = n - c positions: with [lo, hi) the tie group that contains position c, the positives above the
+// group plus the group's positives by their expected share (hi - c) / (hi - lo) of its slots above the cut
+__device__ __forceinline__ double tp_at_k_of(long long P, long long plo, long long phi, int64_t lo, int64_t hi, int64_t c) {
+    return (double)(P - phi) + (double)(phi - plo) * (double)(hi - c) / (double)(hi - lo);
+}
+
+__device__ __forceinline__ double tp_at_k(int64_t n, const float* __restrict__ s_score, const int32_t* __restrict__ pre,
+                                          long long P, int64_t c) {
+    const float x = s_score[c];
+    const int64_t lo = bound(s_score, n, x, false), hi = bound(s_score, n, x, true);
+    return tp_at_k_of(P, pre[lo], hi < n ? (long long)pre[hi] : P, lo, hi, c);
+}
+
 __global__ void __launch_bounds__(MT_NT) k_metrics_final(int64_t n, const float* __restrict__ s_score,
                                                          const int32_t* __restrict__ pre,
                                                          const MetricsBlk* __restrict__ blk, const BestBlk* __restrict__ best,
@@ -377,16 +390,7 @@ __global__ void __launch_bounds__(MT_NT) k_metrics_final(int64_t n, const float*
     out[PCG_MT_TN] = tn;
     out[PCG_MT_FN] = fn;
     out[PCG_MT_AP] = P > 0 ? ap / (double)P : nan("");
-    double rk = nan("");
-    if (P > 0) {                               // K = P: the top P positions are c .. n-1
-        const int64_t c_ = n - P;
-        const float x = s_score[c_];
-        const int64_t lo = bound(s_score, n, x, false), hi = bound(s_score, n, x, true);
-        const long long plo = pre[lo], phi = hi < n ? (long long)pre[hi] : P;
-        const double tpk = (double)(P - phi) + (double)(phi - plo) * (double)(hi - c_) / (double)(hi - lo);
-        rk = tpk / (double)P;
-    }
-    out[PCG_MT_RECALL_AT_K] = rk;
+    out[PCG_MT_RECALL_AT_K] = P > 0 ? tp_at_k(n, s_score, pre, P, n - P) / (double)P : nan("");   // K = P
     out[PCG_MT_BEST_GMEAN] = bg;
     out[PCG_MT_BEST_GMEAN_THRESHOLD] = (double)s_score[bgat];
 }
@@ -447,6 +451,249 @@ __global__ void __launch_bounds__(MT_NT) k_curve_write(int64_t n, const float* _
     }
 }
 
+// ------------------------------------------------------------------------------- operating points
+// pcg_binary_points answers caller-chosen requests from the workspace of the last metrics call:
+//   k_points        CTAs 1 .. nb, one per chunk, kind 2 (partial AUC): every tie group [lo, hi) that starts in the
+//                   chunk adds the ROC segment from (FP(hi)/N, TP(hi)/P) to (FP(lo)/N, TP(lo)/P), clipped at FPR = f,
+//                   as a trapezoid. Thread t owns chunk positions t*MT_PER .. +MT_PER (two 16-byte loads each of
+//                   scores and pre), so a group's hi is the thread's next group start; after the thread's last start it
+//                   is the next thread's first position when that starts a group (distinct scores), else a binary
+//                   search in the chunk's shared scores, or the end of the group that runs past the chunk (one warp
+//                   search per chunk). One fp64
+//                   partial per (request, chunk), part[r * nb + chunk], holding twice the area (the 1/2 of the
+//                   trapezoids is applied once, at the end).
+//                   CTA 0: kinds 0 and 1 and the NaN words of malformed requests, one warp per request (a few
+//                   warp_search calls each), beside the chunk CTAs.
+//   k_points_final  one CTA, kind 2: adds the request's chunk partials in a fixed order and standardises (same bits on
+//                   reruns).
+// Definitions and the output words per kind: include/pcgnn_b200.h.
+
+// The first j in [lo, hi) with !before(j), else hi, for a predicate that holds on a prefix of [lo, hi); called by a
+// whole warp with the same arguments, result in every lane. 32 probes per round: ceil(log32(hi - lo)) dependent loads.
+template <class F>
+__device__ __forceinline__ int64_t warp_search(int64_t lo, int64_t hi, F before) {
+    const int lane = threadIdx.x & 31;
+    while (lo < hi) {
+        const int64_t step = (hi - lo + 31) >> 5;
+        const int64_t p = lo + step * (lane + 1) - 1;
+        const int64_t nlo = lo + step * __popc(__ballot_sync(PCG_FULL, p < hi && before(p)));
+        hi = nlo + step - 1 < hi ? nlo + step - 1 : hi;
+        lo = nlo;
+    }
+    return lo;
+}
+
+__device__ __forceinline__ bool point_valid(int kd, double a, int64_t n) {
+    if (kd == PCG_POINT_TOP_K) return a >= 1.0 && a <= (double)n && a == floor(a);
+    if (kd == PCG_POINT_TPR_AT_FPR) return a >= 0.0 && a <= 1.0;
+    if (kd == PCG_POINT_PAUC) return a > 0.0 && a <= 1.0;
+    return false;
+}
+
+// kinds 0 and 1 (and NaN words for malformed requests other than kind 2), warp w taking requests w, w + 8, ...
+__device__ void points_search(int64_t n, const float* __restrict__ s, const int32_t* __restrict__ pre, long long P,
+                              const int32_t* kd_s, const double* ar_s, int m, double* __restrict__ out) {
+    const long long N = n - P;
+    const double nan_ = nan("");
+    const int lane = threadIdx.x & 31;
+    for (int r = threadIdx.x >> 5; r < m; r += MT_NT / 32) {
+        const int kd = kd_s[r];
+        const double a = ar_s[r];
+        double w[PCG_POINT_WORDS];
+#pragma unroll
+        for (int q = 0; q < PCG_POINT_WORDS; ++q) w[q] = nan_;
+        if (kd == PCG_POINT_PAUC) continue;     // k_points_final (the warp's lanes share r)
+        if (kd == PCG_POINT_TOP_K && point_valid(kd, a, n)) {
+            const int64_t c = n - (int64_t)a;
+            const float x = s[c];
+            const int64_t lo = warp_search(0, c, [&](int64_t j) { return s[j] < x; });
+            const int64_t hi = warp_search(c + 1, n, [&](int64_t j) { return !(x < s[j]); });
+            const double tpk = tp_at_k_of(P, pre[lo], hi < n ? (long long)pre[hi] : P, lo, hi, c);
+            w[0] = P > 0 ? tpk / (double)P : nan_;
+            w[1] = tpk / a;
+            w[2] = (double)x;
+            w[3] = tpk;
+            w[4] = a - tpk;
+        } else if (kd == PCG_POINT_TPR_AT_FPR && point_valid(kd, a, n) && P > 0 && N > 0) {
+            const double lim = a * (double)N;   // FP(j) = (n - j) - (P - pre[j]) does not increase; FP(n) = 0
+            int64_t j = warp_search(0, n, [&](int64_t i) { return (double)((n - i) - (P - pre[i])) > lim; });
+            if (j > 0 && j < n && s[j - 1] == s[j]) {       // inside a tie group: its cut is the next group start
+                const float x = s[j];
+                j = warp_search(j + 1, n, [&](int64_t i) { return !(x < s[i]); });
+            }
+            const long long tp = j < n ? P - pre[j] : 0, fp = (n - j) - tp;
+            w[0] = (double)tp / (double)P;
+            w[1] = (double)fp / (double)N;
+            w[2] = j < n ? (double)s[j] : (double)INFINITY;
+            w[3] = (double)tp;
+            w[4] = (double)fp;
+        }
+        if (lane < PCG_POINT_WORDS) {
+            double v = w[0];
+#pragma unroll
+            for (int q = 1; q < PCG_POINT_WORDS; ++q) v = lane == q ? w[q] : v;
+            out[(size_t)r * PCG_POINT_WORDS + lane] = v;
+        }
+    }
+}
+
+// the requests into shared memory (m <= PCG_POINTS_MAX)
+__device__ __forceinline__ void load_points(const int32_t* __restrict__ kind, const double* __restrict__ arg, int m,
+                                            int* kd_s, double* ar_s) {
+    for (int r = threadIdx.x; r < m; r += MT_NT) {
+        kd_s[r] = kind[r];
+        ar_s[r] = arg[r];
+    }
+}
+
+__global__ void __launch_bounds__(MT_NT, 2) k_points(int64_t n, const float* __restrict__ s_score,
+                                                     const int32_t* __restrict__ s_lab, const int32_t* __restrict__ pre,
+                                                     const int32_t* __restrict__ kind, const double* __restrict__ arg,
+                                                     int m, int nb, double* __restrict__ part, double* __restrict__ out) {
+    __shared__ float sc_s[MT_CH];
+    __shared__ int pf_s[MT_NT];                // pre at each thread's first position
+    __shared__ int kd_s[PCG_POINTS_MAX];
+    __shared__ double ar_s[PCG_POINTS_MAX];
+    __shared__ double red[MT_NT / 32];
+    __shared__ long long edge_hi, edge_tp;
+    const long long P = (long long)pre[n - 1] + (s_lab[n - 1] != 0);
+    load_points(kind, arg, m, kd_s, ar_s);
+    __syncthreads();
+    if (blockIdx.x == 0) {
+        points_search(n, s_score, pre, P, kd_s, ar_s, m, out);
+        return;
+    }
+    const int chunk = (int)blockIdx.x - 1;
+    int any = 0;
+    for (int r = threadIdx.x; r < m; r += MT_NT) any |= kd_s[r] == PCG_POINT_PAUC && point_valid(kd_s[r], ar_s[r], n);
+    if (!__syncthreads_or(any) || P == 0 || P == n) return;   // no partial AUC to compute (NaN: k_points_final)
+    const double iP = 1.0 / (double)P, iN = 1.0 / (double)(n - P);
+    const int64_t j0 = (int64_t)chunk * MT_CH;
+    const int kend = (int)(n - j0 < (int64_t)MT_CH ? n - j0 : (int64_t)MT_CH);
+    const int k0 = threadIdx.x * MT_PER;
+    float sv[MT_PER];                          // the thread's positions k0 .. k0 + MT_PER, straight from global memory
+    int pv[MT_PER];
+    if (k0 + MT_PER <= kend) {                 // 32-byte aligned: chunks start at multiples of MT_CH
+        const float4* s4 = (const float4*)(s_score + j0 + k0);
+        const int4* p4 = (const int4*)(pre + j0 + k0);
+        const float4 a0 = s4[0], a1 = s4[1];
+        const int4 b0 = p4[0], b1 = p4[1];
+        sv[0] = a0.x; sv[1] = a0.y; sv[2] = a0.z; sv[3] = a0.w; sv[4] = a1.x; sv[5] = a1.y; sv[6] = a1.z; sv[7] = a1.w;
+        pv[0] = b0.x; pv[1] = b0.y; pv[2] = b0.z; pv[3] = b0.w; pv[4] = b1.x; pv[5] = b1.y; pv[6] = b1.z; pv[7] = b1.w;
+    } else {
+#pragma unroll
+        for (int u = 0; u < MT_PER; ++u) {
+            sv[u] = k0 + u < kend ? s_score[j0 + k0 + u] : 0.f;
+            pv[u] = k0 + u < kend ? pre[j0 + k0 + u] : 0;
+        }
+    }
+#pragma unroll
+    for (int u = 0; u < MT_PER; ++u) sc_s[k0 + u] = sv[u];
+    pf_s[threadIdx.x] = pv[0];
+    if (threadIdx.x < 32) {                    // the end of the chunk's last group, which may run past the chunk
+        const int64_t e = j0 + kend;
+        const float v = s_score[e - 1];
+        const int64_t hi = e < n && !(v < s_score[e]) ? warp_search(e + 1, n, [&](int64_t j) { return !(v < s_score[j]); })
+                                                      : e;
+        if (threadIdx.x == 0) {
+            edge_hi = hi;
+            edge_tp = hi < n ? P - pre[hi] : 0;
+        }
+    }
+    const float before = k0 == 0 && j0 > 0 ? s_score[j0 - 1] : 0.f;   // thread 0: the previous chunk's last score
+    __syncthreads();
+    double x[MT_PER], y[MT_PER];               // ROC point of the group starting at k0 + u; x < 0: no group start there
+    bool started = false;
+    float v = 0.f;                             // score of the thread's last group start
+#pragma unroll
+    for (int u = 0; u < MT_PER; ++u) {
+        const int k = k0 + u;
+        const float prev = u > 0 ? sv[u - 1] : (k0 > 0 ? sc_s[k0 - 1] : before);
+        x[u] = -1.0;
+        y[u] = 0.0;
+        if (k < kend && (j0 + k == 0 || sv[u] != prev)) {
+            const long long tp = P - pv[u];
+            x[u] = (double)((n - j0 - k) - tp) * iN;
+            y[u] = (double)tp * iP;
+            started = true;
+            v = sv[u];
+        }
+    }
+    double xe = 0.0, ye = 0.0;                 // the point of the group start after the thread's last one
+    if (started) {
+        int a = k0 + MT_PER < kend ? k0 + MT_PER : kend;
+        long long tp;
+        if (a < kend && v < sc_s[a]) {         // the next thread's first position starts a group (distinct scores)
+            tp = P - pf_s[threadIdx.x + 1];
+        } else {                               // first larger score in the chunk, else kend
+            int b = kend;
+            while (a < b) {
+                const int mid = (a + b) >> 1;
+                if (!(v < sc_s[mid])) a = mid + 1; else b = mid;
+            }
+            tp = a < kend ? P - pre[j0 + a] : edge_tp;
+        }
+        const int64_t hi = a < kend ? j0 + a : edge_hi;
+        xe = (double)((n - hi) - tp) * iN;
+        ye = (double)tp * iP;
+    }
+    for (int r = 0; r < m; ++r) {
+        const double f = ar_s[r];
+        if (kd_s[r] != PCG_POINT_PAUC || !point_valid(PCG_POINT_PAUC, f, n)) continue;   // the same for every thread
+        double acc = 0.0, xh = xe, yh = ye;
+#pragma unroll
+        for (int u = MT_PER - 1; u >= 0; --u) {
+            if (x[u] < 0.0) continue;
+            if (xh < f) {
+                if (x[u] <= f) {
+                    acc += (x[u] - xh) * (y[u] + yh);
+                } else {                       // TPR at f on the segment, linearly
+                    const double yf = yh + (y[u] - yh) * (f - xh) / (x[u] - xh);
+                    acc += (f - xh) * (yf + yh);
+                }
+            }
+            xh = x[u];
+            yh = y[u];
+        }
+        acc = block_sum(acc, red);
+        if (threadIdx.x == 0) part[(size_t)r * nb + chunk] = acc;
+    }
+}
+
+__global__ void __launch_bounds__(MT_NT) k_points_final(int64_t n, const int32_t* __restrict__ s_lab,
+                                                        const int32_t* __restrict__ pre, const int32_t* __restrict__ kind,
+                                                        const double* __restrict__ arg, int m, int nb,
+                                                        const double* __restrict__ part, double* __restrict__ out) {
+    __shared__ int kd_s[PCG_POINTS_MAX];
+    __shared__ double ar_s[PCG_POINTS_MAX];
+    __shared__ double red[MT_NT / 32];
+    const long long P = (long long)pre[n - 1] + (s_lab[n - 1] != 0), N = n - P;
+    load_points(kind, arg, m, kd_s, ar_s);
+    __syncthreads();
+    for (int r = 0; r < m; ++r) {
+        if (kd_s[r] != PCG_POINT_PAUC) continue;
+        const double f = ar_s[r];
+        const bool ok = point_valid(PCG_POINT_PAUC, f, n) && P > 0 && N > 0;
+        double acc = 0.0;
+        if (ok) {
+#pragma unroll 4
+            for (int b = threadIdx.x; b < nb; b += MT_NT) acc += part[(size_t)r * nb + b];
+        }
+        acc = block_sum(acc, red);
+        if (threadIdx.x == 0) {
+            double* o = out + (size_t)r * PCG_POINT_WORDS;
+            const double A = 0.5 * acc, lo_area = 0.5 * f * f, nan_ = nan("");
+            o[0] = ok ? 0.5 * (1.0 + (A - lo_area) / (f - lo_area)) : nan_;     // sklearn's McClish correction
+            o[1] = ok ? A : nan_;
+            for (int q = 2; q < PCG_POINT_WORDS; ++q) o[q] = nan_;
+        }
+    }
+}
+
+static size_t points_part_bytes(int64_t n, int m) {
+    return align256((size_t)m * (size_t)((n + MT_CH - 1) / MT_CH) * sizeof(double));
+}
+
 extern "C" size_t pcg_binary_metrics_workspace_bytes(int64_t n) {
     if (n <= 0 || n > 0x7fffffff) return 0;
     return metrics_layout(nullptr, n).total;
@@ -482,4 +729,29 @@ extern "C" int pcg_binary_curve(const void* workspace, size_t workspace_bytes, i
     k_curve_scan<<<1, MT_NT, 0, stream>>>(w.best, nb, count);
     k_curve_write<<<nb, MT_NT, 0, stream>>>(n, w.s_score, w.s_lab, w.pre, w.best, thr, tp, fp);
     return pcg_check_launch("pcg_binary_curve");
+}
+
+extern "C" size_t pcg_binary_points_workspace_bytes(int64_t n, int m) {
+    if (n <= 0 || n > 0x7fffffff || m <= 0 || m > PCG_POINTS_MAX) return 0;
+    return points_part_bytes(n, m);
+}
+
+extern "C" int pcg_binary_points(const void* metrics_ws, size_t metrics_ws_bytes, int64_t n, const int32_t* kind,
+                                 const double* arg, int m, double* out, void* ws, size_t ws_bytes, pcg_stream_t stream_) {
+    cudaStream_t stream = (cudaStream_t)stream_;
+    PCG_REQUIRE(metrics_ws && kind && arg && out && ws, "pcg_binary_points: null pointer");
+    PCG_REQUIRE(n > 0 && n <= 0x7fffffff, "pcg_binary_points: need 0 < n < 2^31 (n=%lld)", (long long)n);
+    PCG_REQUIRE(m > 0 && m <= PCG_POINTS_MAX, "pcg_binary_points: need 0 < m <= %d requests (m=%d)", PCG_POINTS_MAX, m);
+    const MetricsWs w = metrics_layout((char*)metrics_ws, n);
+    PCG_REQUIRE(((uintptr_t)metrics_ws & 255) == 0 && metrics_ws_bytes >= w.total,
+                "pcg_binary_points: metrics_ws must be 256-byte aligned and pcg_binary_metrics_workspace_bytes(n) long");
+    PCG_REQUIRE(((uintptr_t)ws & 7) == 0 && ws_bytes >= points_part_bytes(n, m),
+                "pcg_binary_points: ws must be 8-byte aligned and pcg_binary_points_workspace_bytes(n, m) long");
+    PCG_REQUIRE(((uintptr_t)kind & 3) == 0 && ((uintptr_t)arg & 7) == 0 && ((uintptr_t)out & 7) == 0,
+                "pcg_binary_points: kind, arg and out must be aligned to their element size");
+    const int nb = (int)((n + MT_CH - 1) / MT_CH);
+    double* part = (double*)ws;
+    k_points<<<nb + 1, MT_NT, 0, stream>>>(n, w.s_score, w.s_lab, w.pre, kind, arg, m, nb, part, out);
+    k_points_final<<<1, MT_NT, 0, stream>>>(n, w.s_lab, w.pre, kind, arg, m, nb, part, out);
+    return pcg_check_launch("pcg_binary_points");
 }

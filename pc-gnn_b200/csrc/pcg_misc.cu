@@ -32,7 +32,7 @@ extern "C" int pcg_set_pdl(int enabled) {
     g_pdl = enabled;
     return old;
 }
-extern "C" int pcg_version(void) { return 101; }
+extern "C" int pcg_version(void) { return 102; }
 
 // ------------------------------------------------------------------------------- score table
 // score[v] = <feat[v, :], w> + b. Eight lanes per row, float4 loads, fixed reduction tree (so the

@@ -14,6 +14,7 @@ import numpy as np
 import torch
 
 from . import _lib
+from .metrics import _point_requests, _points_dict
 
 __all__ = ["GraphedTrainStep", "GraphedEvalPass", "pack_eval_plan"]
 
@@ -446,7 +447,13 @@ class GraphedEvalPass:
     the self rows for ``Encoder(gcn=False)``) and the head + to_prob's sigmoid (GCN) or log-softmax (GraphSage); their
     plans are padded with the set's lowest-degree node (``pack_eval_plan``'s indptr). Either writes a planar [2, n]
     buffer, then advances the cursor with a copy of the batch's overflow word into a per-entry array. The metrics graph
-    runs ``pcg_binary_metrics`` and copies the result block and the overflow words to pinned memory.
+    runs ``pcg_binary_metrics`` (with ``operating_points``, then ``pcg_binary_points``) and copies the result block and
+    the overflow words to pinned memory.
+
+    ``operating_points``: None, or a dict with any of the lists ``top_k``, ``fpr`` and ``max_fpr`` of
+    ``metrics.device_operating_points``; ``run()`` then also returns them under ``"operating_points"``. The requests
+    live in device memory read by the recorded graph, so ``set_operating_points`` changes their values without
+    re-recording.
 
     Replays read the current parameter values, so in-place updates (optimizer steps) need nothing; a parameter or the
     feature table moving to new storage, new thresholds (PCALayer) or another engine (an aggregator bound to another
@@ -454,7 +461,7 @@ class GraphedEvalPass:
     left alone. There is no torch fallback: models, tables, graphs and shapes the recorded path does not cover raise
     ``PcgError``."""
 
-    def __init__(self, model, nodes, labels, batch_size: int, cap_slots: int | None = None):
+    def __init__(self, model, nodes, labels, batch_size: int, cap_slots: int | None = None, operating_points=None):
         self._homo = _baseline_parts(model)
         eng = model.inter1.engine() if self._homo is None else self._homo[0]._get_engine()
         plan = pack_eval_plan(nodes, batch_size, None if self._homo is None else eng.graph.indptr[:eng.N + 1])
@@ -467,6 +474,8 @@ class GraphedEvalPass:
         self.model, self.B, self.n = model, int(batch_size), n
         self.n_entries = int(plan.shape[0])
         self._state()                                  # refusals before any allocation
+        self._pt_host = None if operating_points is None else _point_requests(n, **operating_points)
+        m = 0 if self._pt_host is None else len(self._pt_host[0])
         dev = eng.device
         L = _lib.lib()
         self._plan_host = plan
@@ -475,11 +484,16 @@ class GraphedEvalPass:
         self._nodes = torch.empty(self.B, dtype=torch.int32, device=dev)
         self._cursor = torch.zeros(1, dtype=torch.int32, device=dev)
         self._prob = torch.empty((2, n), dtype=torch.float32, device=dev)
-        # [metrics (doubles) | overflow word of every entry]: one block, one copy to the host
-        W = _lib.METRICS_WORDS
-        self._res = torch.zeros(2 * W + self.n_entries, dtype=torch.int32, device=dev)
+        # [metrics (doubles) | operating points (doubles) | overflow word of every entry]: one block, one copy to the host
+        W, self._ovf_at = _lib.METRICS_WORDS, 2 * (_lib.METRICS_WORDS + m * _lib.POINT_WORDS)
+        self._res = torch.zeros(self._ovf_at + self.n_entries, dtype=torch.int32, device=dev)
         self._out = self._res[:2 * W].view(torch.float64)
-        self._ovf = self._res[2 * W:]
+        self._pts = self._res[2 * W:self._ovf_at].view(torch.float64)
+        self._ovf = self._res[self._ovf_at:]
+        if m:
+            self._pt_kind = torch.from_numpy(self._pt_host[0]).to(dev)
+            self._pt_arg = torch.from_numpy(self._pt_host[1]).to(dev)
+            self._pt_ws = torch.empty(int(L.pcg_binary_points_workspace_bytes(n, m)), dtype=torch.uint8, device=dev)
         self._pin = torch.zeros(self._res.numel(), dtype=torch.int32, pin_memory=True)
         self._pin_np = self._pin.numpy()
         self._mws = torch.empty(int(L.pcg_binary_metrics_workspace_bytes(n)), dtype=torch.uint8, device=dev)
@@ -635,6 +649,11 @@ class GraphedEvalPass:
         L = _lib.lib()
         _lib.check(L.pcg_binary_metrics(self._prob.data_ptr(), self._labels.data_ptr(), self.n, self._out.data_ptr(),
                                         self._mws.data_ptr(), self._mws.numel(), _lib.stream_ptr()), "pcg_binary_metrics")
+        if self._pt_host is not None:
+            _lib.check(L.pcg_binary_points(self._mws.data_ptr(), self._mws.numel(), self.n, self._pt_kind.data_ptr(),
+                                           self._pt_arg.data_ptr(), len(self._pt_host[0]), self._pts.data_ptr(),
+                                           self._pt_ws.data_ptr(), self._pt_ws.numel(), _lib.stream_ptr()),
+                       "pcg_binary_points")
         _lib.check(L.pcg_stage(self._res.data_ptr(), _lib.host_device_ptr(self._pin), self._res.numel() * 4,
                                _lib.stream_ptr()), "pcg_stage")
 
@@ -645,6 +664,9 @@ class GraphedEvalPass:
         The metrics are computed on ``probs()`` as they are: for GraphSage, log-probabilities, so ``best_threshold``
         and ``best_gmean_threshold`` are log-probabilities there (pred, AUC and the ranking keys ap, recall_at_k,
         best_f1_macro and best_gmean need no conversion: log is monotone).
+        A pass built with ``operating_points`` adds the key ``"operating_points"`` (``metrics.device_operating_points``'
+        result for the current requests, computed in the same metrics graph); for GraphSage its thresholds are
+        log-probabilities too, its counts and rates need no conversion.
         Raises PcgError when a batch needed more slots than ``cap_slots`` (its scores would be incomplete)."""
         key = self._state()
         if key != self._key:
@@ -659,11 +681,26 @@ class GraphedEvalPass:
         self._done.record(torch.cuda.current_stream(self._prob.device))
         self._done.synchronize()
         W = _lib.METRICS_WORDS
-        bad = np.flatnonzero(self._pin_np[2 * W:])
+        bad = np.flatnonzero(self._pin_np[self._ovf_at:])
         if bad.size:
             raise _lib.PcgError(f"GraphedEvalPass: {bad.size} of {self.n_entries} batches needed more than cap_slots="
                                 f"{self.cap_slots} slots (first: entry {int(bad[0])}); build the pass with a larger capacity")
-        return dict(zip(_lib.METRICS_KEYS, self._pin_np[:2 * W].view(np.float64).tolist()))
+        res = dict(zip(_lib.METRICS_KEYS, self._pin_np[:2 * W].view(np.float64).tolist()))
+        if self._pt_host is not None:
+            res["operating_points"] = _points_dict(self._pin_np[2 * W:self._ovf_at].view(np.float64), *self._pt_host)
+        return res
+
+    def set_operating_points(self, top_k=(), fpr=(), max_fpr=()):
+        """New values for the requests of a pass built with ``operating_points``, the same number of each kind (the
+        recorded graph reads them from device memory: no re-recording). Used from the next ``run()`` on."""
+        if self._pt_host is None:
+            raise _lib.PcgError("GraphedEvalPass.set_operating_points: the pass was built without operating_points")
+        kind, arg = _point_requests(self.n, top_k, fpr, max_fpr)
+        if not np.array_equal(kind, self._pt_host[0]):
+            raise ValueError("GraphedEvalPass.set_operating_points: needs as many top_k, fpr and max_fpr requests as the "
+                             "pass was built with (build a new pass for other counts)")
+        self._pt_arg.copy_(torch.from_numpy(arg))
+        self._pt_host = (kind, arg)
 
     def curve(self) -> tuple:
         """ROC / PR curve of the last ``run()`` (``metrics.device_curve`` of ``probs()``): (thresholds fp32 [G],
